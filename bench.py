@@ -5,10 +5,11 @@ A "step" is one pass of the hot path over the whole synthetic structured-tet duc
 fused Jacobian + residual assembly (incl. lifting, BC rows/cols, BC diagonal, set_bc), i.e. what
 NonlinearPDE_SNESProblem.J + .F do at one Newton iterate (NavierStokes/NavierStokesChannelFlow.py:51-75).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload L|M|S] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload L|M|S] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); the duct is cut into x-slabs (strong scaling: the total
 mesh is fixed).  One JSON line is printed by rank 0.  See DESIGN.md "Measurement" for the byte model.
+--dump-outputs DIR (1 GPU) writes what the last timed step computed to DIR/*.npy (see dump_outputs).
 """
 import argparse
 import json
@@ -157,6 +158,36 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------- our arm
+DUMP_MAX_ENTRIES = 1 << 21      # per dumped array: 16 MB of float64
+
+
+def dump_outputs(asm, F_dev, out_dir):
+    """Write what one step hands its caller to out_dir as float64 .npy files: residual.npy, the residual F of the owned rows,
+    and jacobian_values.npy, the CSR values of J in the caller's row order.  An output longer than DUMP_MAX_ENTRIES is cut to
+    a fixed sample: F at seeded positions, J as whole rows in seeded blocks of 256 consecutive rows.  The bench's inputs are
+    seeded as well, so two builds of the project can be compared entry for entry."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(7)
+    n = asm.n_owned
+    F = np.empty(n)
+    asm.d2h(F, F_dev)
+    if n > DUMP_MAX_ENTRIES:
+        F = F[np.sort(rng.choice(n, DUMP_MAX_ENTRIES, replace=False))]
+    vals_dev = asm.values_dev()
+    if asm.nnz <= DUMP_MAX_ENTRIES:
+        J = asm.get_value_range(0, asm.nnz, vals_dev)
+    else:
+        block = 256
+        n_blocks = max(1, DUMP_MAX_ENTRIES * n // asm.nnz // block)          # about DUMP_MAX_ENTRIES values in all
+        first = block * np.sort(rng.choice(n // block, n_blocks, replace=False))
+        start, ptr, _ = asm.get_rows(np.concatenate([first, first + block - 1]))
+        last = np.arange(n_blocks) + n_blocks                                # positions of the blocks' last rows
+        end = start[last] + ptr[last + 1] - ptr[last]
+        J = np.concatenate([asm.get_value_range(b, e - b, vals_dev) for b, e in zip(start[:n_blocks], end)])
+    np.save(os.path.join(out_dir, "residual.npy"), F)
+    np.save(os.path.join(out_dir, "jacobian_values.npy"), J)
+
+
 def run_ours(args):
     from stabilized_navier_stokes_flow_fenicsx_b200 import mesh as M
     from stabilized_navier_stokes_flow_fenicsx_b200.assembler import NSAssembler
@@ -165,6 +196,8 @@ def run_ours(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a one-GPU run: every rank holds only its slab of the outputs")
     comm = D.Comm.from_env() if world > 1 else D.Comm.single()
     n_cross, n_long = WORKLOADS[args.workload]
 
@@ -218,6 +251,8 @@ def run_ours(args):
     launches = asm.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     ms_per_step = comm.max(total_ms / args.steps)
+    if args.dump_outputs:
+        dump_outputs(asm, F_dev, args.dump_outputs)
 
     # dominant kernel alone (CUDA events on the library's stream around the assembly kernel), timed live
     kms = []
@@ -440,7 +475,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the small P2-P1 / streamline-tracer measurements (other_paths)")
     ap.add_argument("--no-aij", action="store_true", help="skip the AIJ-mode end-to-end step (values to pinned host memory)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the residual and Jacobian values of the last timed step to DIR/*.npy (1 GPU; sampled above 2^21 entries)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
