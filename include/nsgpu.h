@@ -38,7 +38,8 @@ enum {
   NSGPU_EUNSUPPORTED = -3,
   NSGPU_ENCCL = -4,
   NSGPU_EPATTERN = -5, /* element entry outside the sparsity pattern / row too long */
-  NSGPU_ENONFINITE = -6 /* the assembled residual holds NaN / Inf (diverged state or degenerate cell); see option "check_finite" */
+  NSGPU_ENONFINITE = -6, /* the assembled residual holds NaN / Inf (diverged state or degenerate cell); see option "check_finite" */
+  NSGPU_EZEROPIVOT = -7  /* the point ILU(0) factorisation met a zero or non-finite pivot (PETSc: factor zero-pivot failure) */
 };
 
 /* weak-form flavours (nsgpu_set_form) */
@@ -119,7 +120,9 @@ int nsgpu_spmv(nsgpu_ctx* ctx, const double* x_local, double* y_owned);
  * Jacobian of the last nsgpu_jacobian*: transpose-free QMR, right-preconditioned, every vector and scalar
  * device-resident; two MatMults per iteration, dot products reduced over all ranks (ncclAllReduce).
  *   pc: 0 none, 1 Jacobi, 4 = 4x4 block Jacobi over the dofs of one P1-P1 vertex (falls back to 1 elsewhere),
- *       5 = multicolour 4x4-block ILU(0), block Jacobi over the ranks (P1-P1 tets; NSGPU_EUNSUPPORTED elsewhere).
+ *       5 = multicolour 4x4-block ILU(0), block Jacobi over the ranks (P1-P1 tets; NSGPU_EUNSUPPORTED elsewhere),
+ *       6 = multicolour point ILU(0), block Jacobi over the ranks, any space (velocity dofs eliminated before pressure dofs;
+ *           NSGPU_EZEROPIVOT on a zero pivot).
  *   zero_guess != 0 ignores the incoming x (PETSc's default initial guess).
  * Stops when the quasi-residual bound tau*sqrt(m+1) <= max(rtol * ||b||, atol) (PETSc's default test) or after max_it iterations;
  * *its_out = iterations done, *rnorm_out = TRUE residual norm ||b - A x|| at exit, *r0norm_out = ||b - A x0||.
@@ -137,6 +140,16 @@ int nsgpu_tfqmr_dev(nsgpu_ctx* ctx, const double* b_owned_dev, double* x_local_d
  * (= the caller's order when its numbering is vertex-blocked, dof = 4 vertex + component) and the number of colours; for tests. */
 int nsgpu_ilu_apply(nsgpu_ctx* ctx, int refactor, const double* r_owned, double* z_owned);
 int nsgpu_ilu_colours(nsgpu_ctx* ctx, int32_t* colour /* n_owned / 4, may be NULL */, int32_t* n_colours);
+/* Multicolour point ILU(0) of the resident Jacobian (pc = 6 of nsgpu_tfqmr*): PETSc's default PC on the AIJ matrix of the mixed space
+ * (block size 1), block Jacobi over the ranks.  The owned dofs are coloured on the graph of the CSR pattern, velocity dofs first and
+ * pressure dofs with colours numbered after every velocity colour, and eliminated in the order (colour, row): every pressure pivot
+ * then carries the local Schur complement, so the unstabilised Taylor-Hood Stokes operator (zero pressure diagonal) factorises.
+ * nsgpu_pilu_apply = PCApply on host vectors in the caller's numbering: z = U^-1 L^-1 r; refactor != 0 factorises the current values
+ * first (always done when there is no factorisation yet); NSGPU_EZEROPIVOT names the row of a zero pivot.  nsgpu_pilu_colours: the
+ * elimination colour of every owned dof in the caller's numbering, the number of colours and how many of them are velocity colours
+ * (within a colour the order does not change the factor); for tests. */
+int nsgpu_pilu_apply(nsgpu_ctx* ctx, int refactor, const double* r_owned, double* z_owned);
+int nsgpu_pilu_colours(nsgpu_ctx* ctx, int32_t* colour /* n_owned, may be NULL */, int32_t* n_colours, int32_t* n_velocity_colours);
 int nsgpu_axpy_dev(nsgpu_ctx* ctx, double a, const double* x_dev, double* y_dev);
 int nsgpu_norm_dev(nsgpu_ctx* ctx, const double* x_dev, double* out);
 /* VecDot over the owned entries, reduced over all ranks (the initial slope F . J dx of SNES' backtracking line search). */

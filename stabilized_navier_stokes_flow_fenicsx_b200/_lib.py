@@ -45,6 +45,8 @@ SIGNATURES = {
                                        ctypes.POINTER(ctypes.c_int), c_f64p, c_f64p]),
     "nsgpu_ilu_apply": (ctypes.c_int, [c_ctx, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]),
     "nsgpu_ilu_colours": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.POINTER(ctypes.c_int32)]),
+    "nsgpu_pilu_apply": (ctypes.c_int, [c_ctx, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]),
+    "nsgpu_pilu_colours": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]),
     "nsgpu_axpy_dev": (ctypes.c_int, [c_ctx, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
     "nsgpu_norm_dev": (ctypes.c_int, [c_ctx, ctypes.c_void_p, c_f64p]),
     "nsgpu_dot_dev": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.c_void_p, c_f64p]),

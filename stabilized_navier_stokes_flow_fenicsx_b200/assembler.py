@@ -203,6 +203,8 @@ class NSAssembler:
 
     def tfqmr(self, b, x0=None, rtol=1e-8, atol=0.0, max_it=1000, pc=4):
         """KSPSolve with KSPTFQMR on the resident Jacobian (NavierStokesChannelFlow.py:77, :282-285), fully on the device.
+        pc: 0 none, 1 Jacobi, 4 4x4 vertex-block Jacobi (P1-P1 tets, else 1), 5 multicolour block ILU(0) (P1-P1 tets only),
+        6 multicolour point ILU(0) (any space; NsgpuError "zero pivot" when a pivot vanishes).
         Returns (x_owned, info) with info = dict(its, rnorm = true ||b - A x||, r0norm)."""
         b = np.ascontiguousarray(b, dtype=np.float64)
         x = np.zeros(self.n_owned) if x0 is None else np.array(x0[: self.n_owned], dtype=np.float64)
@@ -212,6 +214,7 @@ class NSAssembler:
         return x, {"its": its.value, "rnorm": rn.value, "r0norm": r0.value}
 
     def tfqmr_dev(self, b_dev, x_dev, rtol=1e-8, atol=0.0, max_it=1000, pc=4, zero_guess=True):
+        """``tfqmr`` on device vectors (b: n_owned, x: n_cols doubles); pc as in ``tfqmr``."""
         its, rn, r0 = ctypes.c_int(), ctypes.c_double(), ctypes.c_double()
         self._check(self.lib.nsgpu_tfqmr_dev(self.ctx, b_dev, x_dev, float(rtol), float(atol), int(max_it), int(pc), 1 if zero_guess else 0,
                                              ctypes.byref(its), ctypes.byref(rn), ctypes.byref(r0)), "tfqmr_dev")
@@ -233,6 +236,23 @@ class NSAssembler:
         self._check(self.lib.nsgpu_ilu_colours(self.ctx, _ptr(col), ctypes.byref(n)), "ilu_colours")
         return col, n.value
 
+    def pilu_apply(self, r, refactor=True):
+        """PCApply of the multicolour point ILU(0) (pc = 6) on a host vector in the caller's numbering: z = U^-1 L^-1 r (owned entries)."""
+        r = np.ascontiguousarray(r, dtype=np.float64)
+        if r.size < self.n_owned:
+            raise ValueError(f"pilu_apply needs the {self.n_owned} owned entries")
+        z = np.empty(self.n_owned)
+        self._check(self.lib.nsgpu_pilu_apply(self.ctx, 1 if refactor else 0, _ptr(r), _ptr(z)), "pilu_apply")
+        return z
+
+    def pilu_colours(self):
+        """(elimination colour per owned dof in the caller's numbering, number of colours, number of velocity colours); the
+        velocity colours are 0 .. n_velocity_colours - 1, the pressure colours come after them."""
+        n, nv = ctypes.c_int32(), ctypes.c_int32()
+        col = np.empty(self.n_owned, dtype=np.int32)
+        self._check(self.lib.nsgpu_pilu_colours(self.ctx, _ptr(col), ctypes.byref(n), ctypes.byref(nv)), "pilu_colours")
+        return col, n.value, nv.value
+
     def axpy_dev(self, a, x_dev, y_dev):
         self._check(self.lib.nsgpu_axpy_dev(self.ctx, float(a), x_dev, y_dev), "axpy_dev")
 
@@ -251,7 +271,8 @@ class NSAssembler:
         NavierStokesChannelFlow.py:286-291): F and J from the assembly kernels, dw from TFQMR, w -= lambda dw.
         ``linesearch``: "bt" = PETSc's default for newtonls (SNESLineSearchBT: sufficient decrease alpha = 1e-4 on
         1/2 ||F||^2, quadratic then cubic backtracking, steps clipped to [0.1, 0.5] of the previous one, at most 40), or
-        "basic" (full steps).  Nothing but a few scalars crosses PCIe.  w_dev: n_cols doubles (state in / solution out)."""
+        "basic" (full steps).  ``pc``: the preconditioner of the TFQMR solves, as in ``tfqmr`` (6, the point ILU(0), works on every
+        space).  Nothing but a few scalars crosses PCIe.  w_dev: n_cols doubles (state in / solution out)."""
         nbytes = 8 * self.n_cols
         owns = work is None
         F_dev, dw_dev = (self.dev_alloc(nbytes), self.dev_alloc(nbytes)) if owns else work[:2]

@@ -82,6 +82,7 @@ struct nsgpu_ctx {
   struct nsgpu_p1tet_plan* p1plan = nullptr;   // factorised P1-P1 tet kernels (p1tet.cu)
   void* krylov = nullptr;                      // work vectors of the device-resident TFQMR (krylov.cu)
   void* ilu = nullptr;                         // colouring + factors of the multicolour block ILU(0) preconditioner (ilu.cu)
+  void* pilu = nullptr;                        // colouring + factor of the multicolour point ILU(0) preconditioner (pilu.cu)
   void* rowown_plan = nullptr;                 // entity incidence lists + point records of the row-owner kernel (rowown.cu)
   void* trace = nullptr;                       // locator + velocity tables of the streamline tracer (streamtrace.cu)
 
@@ -213,6 +214,12 @@ int ilu_factor(nsgpu_ctx* ctx);
 int ilu_apply(nsgpu_ctx* ctx, const double* d_r, double* d_z);
 int ilu_colours(nsgpu_ctx* ctx, int32_t* h_colour, int32_t* n_colours);
 void ilu_free(nsgpu_ctx* ctx);
+// pilu.cu
+int pilu_factor(nsgpu_ctx* ctx);
+bool pilu_factored(const nsgpu_ctx* ctx);
+int pilu_apply(nsgpu_ctx* ctx, const double* d_r, double* d_z);
+int pilu_colours(nsgpu_ctx* ctx, int32_t* h_colour, int32_t* n_colours, int32_t* n_vel_colours);
+void pilu_free(nsgpu_ctx* ctx);
 // rowown.cu
 bool rowown_available(nsgpu_ctx* ctx);
 int rowown_assemble(nsgpu_ctx* ctx, const double* d_xin, bool want_J, bool want_F, double* d_Fout);

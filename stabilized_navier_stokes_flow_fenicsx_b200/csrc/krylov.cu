@@ -5,7 +5,7 @@
 // products, and (b) Newton can be driven to convergence in containers without PETSc (tests: converged-solution parity).
 //
 // Algorithm: Freund's transpose-free QMR in the two-half-step form (C.T. Kelley, "Iterative Methods for Linear and
-// Nonlinear Equations", SIAM 1995, algorithm tfqmr), RIGHT-preconditioned with (block-)Jacobi: A M^-1 y = b, x = M^-1 y,
+// Nonlinear Equations", SIAM 1995, algorithm tfqmr), RIGHT-preconditioned (Jacobi, block Jacobi, block or point ILU(0)): A M^-1 y = b, x = M^-1 y,
 // so the quasi-residual bound tau * sqrt(m + 1) refers to the true residual.  All scalars (rho, alpha, tau, theta, eta, ...)
 // live in device memory and are updated by one-thread "finalize" kernels; the host only reads the bound once per
 // iteration to decide whether to stop.  Every vector update is fused with the reduction that follows it.
@@ -285,6 +285,7 @@ static int reduce_and_update(nsgpu_ctx* ctx, Work& k, int nblocks, int what) {
 // out (n_owned) = A M^-1 y
 static int pc_apply(nsgpu_ctx* ctx, Work& k, int bs, const double* y, double* t) {
   if (bs == 5) return ilu_apply(ctx, y, t);                       // multicolour block ILU(0), ilu.cu
+  if (bs == 6) return pilu_apply(ctx, y, t);                      // multicolour point ILU(0), pilu.cu
   const bool wide = bs == 4 && ((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(k.dinv)) & 31) == 0;
   k_pc_apply<<<(unsigned)ceil_div(k.n > 0 ? k.n : 1, 256), 256, 0, ctx->stream>>>(k.n, bs, k.dinv, y, t, wide);
   ctx->launches += 1;
@@ -313,9 +314,14 @@ int tfqmr_impl(nsgpu_ctx* ctx, const double* d_b, double* d_x, double rtol, doub
   const unsigned g = vgrid(n);
   int bs = pc;
   if (bs == 4 && (n % 4 != 0 || ctx->gdim != 3 || ctx->vdeg != 1)) bs = 1;   // vertex blocks only exist for P1-P1 tets
-  if (bs != 0 && bs != 1 && bs != 4 && bs != 5) { set_error(ctx, "tfqmr: pc must be 0 (none), 1 (Jacobi), 4 (4x4 block Jacobi) or 5 (multicolour block ILU(0))"); return NSGPU_EINVAL; }
+  if (bs != 0 && bs != 1 && bs != 4 && bs != 5 && bs != 6) {
+    set_error(ctx, "tfqmr: pc must be 0 (none), 1 (Jacobi), 4 (4x4 block Jacobi), 5 (multicolour block ILU(0)) or 6 (multicolour point ILU(0))");
+    return NSGPU_EINVAL;
+  }
   if (bs == 5) {
     if ((rc = ilu_factor(ctx))) return rc;
+  } else if (bs == 6) {
+    if ((rc = pilu_factor(ctx))) return rc;
   } else if (bs) {
     const int64_t ne = bs == 4 ? n / 4 : n;
     k_pc_setup<<<(unsigned)ceil_div(ne > 0 ? ne : 1, 128), 128, 0, s>>>(n, bs, ctx->d_indptr, ctx->d_indices, ctx->d_diag, ctx->d_vals, k.dinv);

@@ -151,6 +151,7 @@ int nsgpu_destroy(nsgpu_ctx* ctx) {
   p1tet_free(ctx);
   krylov_free(ctx);
   ilu_free(ctx);
+  pilu_free(ctx);
   rowown_free(ctx);
   trace_free(ctx);
   renumber_free(ctx);
@@ -579,6 +580,25 @@ int nsgpu_ilu_apply(nsgpu_ctx* ctx, int refactor, const double* r_owned, double*
 int nsgpu_ilu_colours(nsgpu_ctx* ctx, int32_t* colour, int32_t* n_colours) {
   NS_ENTER(ctx);
   return ilu_colours(ctx, colour, n_colours);
+}
+
+int nsgpu_pilu_apply(nsgpu_ctx* ctx, int refactor, const double* r_owned, double* z_owned) {
+  NS_ENTER(ctx);
+  NS_REQUIRE(ctx, ctx->pattern_built, "pilu_apply: call build_pattern and assemble a Jacobian first");
+  NS_REQUIRE(ctx, r_owned && z_owned, "pilu_apply: NULL argument");
+  int rc;
+  if ((refactor || !pilu_factored(ctx)) && (rc = pilu_factor(ctx))) return rc;
+  if ((rc = vec_in(ctx, r_owned, ctx->d_F, ctx->n_owned))) return rc;
+  if ((rc = pilu_apply(ctx, ctx->d_F, ctx->d_F))) return rc;
+  if ((rc = vec_out(ctx, ctx->d_F, z_owned, ctx->n_owned))) return rc;
+  NS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return NSGPU_OK;
+}
+
+int nsgpu_pilu_colours(nsgpu_ctx* ctx, int32_t* colour, int32_t* n_colours, int32_t* n_velocity_colours) {
+  NS_ENTER(ctx);
+  NS_REQUIRE(ctx, ctx->pattern_built, "pilu_colours: call build_pattern first");
+  return pilu_colours(ctx, colour, n_colours, n_velocity_colours);
 }
 
 int nsgpu_axpy_dev(nsgpu_ctx* ctx, double a, const double* x_dev, double* y_dev) {

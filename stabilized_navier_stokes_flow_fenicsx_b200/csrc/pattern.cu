@@ -345,6 +345,7 @@ int build_pattern_impl(nsgpu_ctx* ctx) {
   p1tet_free(ctx);   // any previous plan refers to the old pattern
   rowown_free(ctx);
   ilu_free(ctx);
+  pilu_free(ctx);
   cleanup();
   if (bad) {
     set_error(ctx, "build_pattern: a cell dof is missing from its row, or a row holds more than 65535 entries");
