@@ -119,8 +119,6 @@ struct nsgpu_ctx {
   int64_t fused_hits = 0;
   int check_finite = 1;    // scan the owned residual entries for NaN / Inf after every residual assembly (status NSGPU_ENONFINITE)
   int* d_nonfinite = nullptr;
-  bool ilu_factor16 = true; // multicolour ILU: sixteen lanes per vertex in the factorisation when no block row is longer than 16
-  bool ilu_packed = true;  // multicolour ILU: keep a second copy of the factor in elimination order (streaming sweeps) when the memory is there
   bool spmv_wide = true;   // vertex-blocked SpMV: 256-bit loads + 4-byte block columns when rows and vectors are 32-byte aligned
   int spmv_blocks = 5;     // vertex-blocked SpMV: resident 256-thread CTAs per SM the kernel is compiled for (4, 5 or 6)
   int stream_chunks = 16;  // tile chunks of the streamed host path
@@ -209,6 +207,13 @@ int norm_impl(nsgpu_ctx* ctx, const double* d_x, double* out);
 int norm_n_impl(nsgpu_ctx* ctx, const double* d_x, int64_t n, double* out);
 int dot_impl(nsgpu_ctx* ctx, const double* d_x, const double* d_y, double* out);
 void krylov_free(nsgpu_ctx* ctx);
+// colour.cu: Jones-Plassmann colouring and elimination order of nodes 0..n-1 for the multicolour ILU(0) preconditioners.  Node e's
+// neighbours are the columns j of CSR row (e << shift), as j >> shift, skipping j >> shift >= n and e itself.  d_cls == nullptr: one
+// class; otherwise (0 / 1 per node) class 0 is coloured first, then class 1 from the first colour after class 0's.  d_order gets the
+// nodes sorted by (colour, node), cstart the n_colours + 1 offsets of the colours in it.  NSGPU_EUNSUPPORTED (before anything is
+// ordered) when the graph needs more than max_colours colours or the rounds run out; messages start with who.
+int mc_colour(nsgpu_ctx* ctx, int64_t n, int shift, const uint8_t* d_cls, int max_colours, const char* who, int32_t* d_colour,
+              int32_t* d_order, std::vector<int64_t>& cstart, int* n_class0_colours);
 // ilu.cu
 int ilu_factor(nsgpu_ctx* ctx);
 int ilu_apply(nsgpu_ctx* ctx, const double* d_r, double* d_z);

@@ -7,12 +7,14 @@
 // colour share no matrix entry, so a colour is factorised, and later substituted, by one kernel launch with one thread group
 // per vertex.  Couplings to other ranks' vertices are dropped (block Jacobi over the ranks, as PETSc does).
 //
-//   colouring   Jones-Plassmann with hashed priorities on the vertex graph of the owned rows (deterministic), <= 64 colours
+//   colouring   Jones-Plassmann with hashed priorities on the vertex graph of the owned rows (deterministic), <= 64 colours: the
+//               routine pc = 6 uses too (colour.cu), on CSR row 4e of vertex e
 //   order       elimination order = (colour, vertex)
 //   factorise   for colour c, vertex i:  for every neighbour k with colour < c, in elimination order:
 //                   L_ik = A_ik U_kk^-1 ;  A_ij -= L_ik U_kj  for the blocks (i, j) of the pattern with j after k    [ILU(0)]
 //               then U_ii^-1 by Gauss-Jordan with partial pivoting
-//   apply       z = U^-1 L^-1 r: one launch per colour forwards (unit lower factor), one per colour backwards
+//   apply       z = U^-1 L^-1 r: one launch per colour forwards (unit lower factor), one per colour backwards, on a packed copy of
+//               the factor in elimination order
 //
 // Block access is the vertex-blocked view the block SpMV uses (p1tet.cu): per vertex the list of neighbour vertices
 // (ctx->d_pairs) and the CSR starts of its four rows, blocks of four contiguous values per row.
@@ -28,8 +30,7 @@ struct IluPlan {
   int n_colours = 0;
   int32_t* d_colour = nullptr;     // per owned vertex
   int32_t* d_order = nullptr;      // vertices sorted by (colour, vertex)
-  int4* d_orec = nullptr;          // per position of the order: (vertex, neighbours, first pair lo, hi): one load instead of order -> pair0 / ns
-  // packed factor (streaming sweeps): the off-diagonal blocks in elimination order -- per position of the order the L blocks (lower
+  // packed factor (what the sweeps read): the off-diagonal blocks in elimination order -- per position of the order the L blocks (lower
   // colour) then the U blocks (higher colour) of its vertex, the column vertex inline -- refilled from d_lu after every factorisation
   int4* d_erec = nullptr;          // per position: (vertex, nL | nU << 16, first packed block lo, hi)
   uint32_t* d_emap = nullptr;      // packed block -> pair index (its source in d_lu)
@@ -40,81 +41,11 @@ struct IluPlan {
   std::vector<int64_t> cstart;     // n_colours + 1 offsets into d_order
   double* d_lu = nullptr;          // 16 doubles per (vertex, neighbour) pair, row-major 4x4, indexed like ctx->d_pairs
   double* d_dinv = nullptr;        // 16 doubles per vertex: U_ii^-1
-  uint8_t* d_nbc = nullptr;        // per (vertex, neighbour) pair: colour of the neighbour (255: other rank's vertex, 254: the vertex itself)
-  bool unsupported = false;
 };
-
-__device__ __forceinline__ uint32_t ilu_hash(uint32_t x) {
-  x ^= x >> 16; x *= 0x7feb352du; x ^= x >> 15; x *= 0x846ca68bu; x ^= x >> 16;
-  return x;
-}
 
 __global__ void k_ilu_check(int64_t nv, const int32_t* __restrict__ rowdof, int* bad) {
   const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (e < nv && rowdof[4 * e] != (int32_t)(4 * e)) *bad = 1;
-}
-
-// one Jones-Plassmann round: an uncoloured vertex whose priority beats every uncoloured neighbour takes the lowest free colour
-__global__ void k_ilu_colour(int64_t nv, int64_t n_owned, const int64_t* __restrict__ pair0, const int32_t* __restrict__ ns,
-                             const uint64_t* __restrict__ pairs, const int32_t* __restrict__ colour, int32_t* colour_out, unsigned long long* left,
-                             int* too_many) {
-  // decisions are taken on the colours at the start of the round (colour), results go to colour_out: the colouring does not
-  // depend on the order in which the threads run
-  const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (e >= nv || colour[e] >= 0) return;
-  const uint32_t pe = ilu_hash((uint32_t)e);
-  unsigned long long used = 0;
-  const int64_t p0 = pair0[e];
-  const int n = ns[e];
-  for (int s = 0; s < n; ++s) {
-    const int64_t B = (int64_t)(pairs[p0 + s] & 0xffffffffu);
-    if (B >= n_owned) continue;
-    const int64_t k = B >> 2;
-    if (k == e) continue;
-    const int ck = colour[k];
-    if (ck >= 0) { used |= 1ull << ck; continue; }
-    const uint32_t pk = ilu_hash((uint32_t)k);
-    if (pk > pe || (pk == pe && k > e)) { atomicAdd(left, 1ull); return; }   // a neighbour goes first
-  }
-  int c = 0;
-  while (c < 64 && ((used >> c) & 1ull)) ++c;
-  if (c >= 64) { *too_many = 1; c = 63; }
-  colour_out[e] = c;
-}
-
-__global__ void k_ilu_keys(int64_t nv, const int32_t* __restrict__ colour, uint64_t* keys) {
-  const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (e < nv) keys[e] = ((uint64_t)(uint32_t)colour[e] << 32) | (uint64_t)e;
-}
-
-__global__ void k_ilu_order(int64_t nv, const uint64_t* __restrict__ keys, int32_t* order, unsigned long long* count) {
-  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (i >= nv) return;
-  order[i] = (int32_t)(keys[i] & 0xffffffffu);
-  atomicAdd(count + (keys[i] >> 32), 1ull);
-}
-
-// neighbour colours next to the neighbour lists: the substitution sweeps read them in a stream instead of gathering colour[]
-__global__ void k_ilu_nbc(int64_t nv, int64_t n_owned, const int64_t* __restrict__ pair0, const int32_t* __restrict__ ns,
-                          const uint64_t* __restrict__ pairs, const int32_t* __restrict__ colour, uint8_t* __restrict__ nbc) {
-  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  const int64_t e = t >> 4;
-  if (e >= nv) return;
-  const int64_t p0 = pair0[e];
-  const int n = ns[e];
-  for (int s = (int)(t & 15); s < n; s += 16) {
-    const int64_t B = (int64_t)(pairs[p0 + s] & 0xffffffffu);
-    nbc[p0 + s] = B >= n_owned ? 255 : ((B >> 2) == e ? 254 : (uint8_t)colour[B >> 2]);
-  }
-}
-
-// the sweeps' per-vertex record in elimination order
-__global__ void k_ilu_orec(int64_t nv, const int32_t* __restrict__ order, const int64_t* __restrict__ pair0, const int32_t* __restrict__ ns, int4* __restrict__ orec) {
-  const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (idx >= nv) return;
-  const int32_t i = order[idx];
-  const int64_t p0 = pair0[i];
-  orec[idx] = make_int4(i, ns[i], (int)(p0 & 0xffffffffLL), (int)(p0 >> 32));
 }
 
 // LU blocks <- the owned x owned blocks of the assembled Jacobian
@@ -375,125 +306,44 @@ __global__ void k_ilu_maxns(int64_t nv, const int32_t* __restrict__ ns, int* out
   if (e < nv) atomicMax(out, ns[e]);
 }
 
-// one colour of the forward (LOWER: z_i -= sum over earlier neighbours L_ik z_k) or backward (z_i = U_ii^-1 (z_i - sum over later
-// neighbours U_ij z_j)) substitution, in place.  Sixteen lanes per vertex.
-// WIDE (32-byte aligned factor and vector): four lanes per block -- lane (slot, r) loads row r of the block of neighbour slot, slot + 4, ...
-// with one 256-bit load, so that one load instruction of the four lanes asks for the whole 128-byte block at once -- and the row
-// sums are reduced over the four slots.  Otherwise: lane s takes neighbour s with scalar loads.
-template <bool LOWER, bool WIDE>
-__global__ void __launch_bounds__(256)
-k_ilu_sweep(int64_t i0, int64_t i1, int cc, const int4* __restrict__ orec, const uint8_t* __restrict__ nbc,
-            const uint64_t* __restrict__ pairs, const double* __restrict__ lu, const double* __restrict__ dinv, double* z) {
-  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  const int64_t idx = i0 + (t >> 4);
-  const int lane = (int)(t & 15);
-  int64_t i = 0;
-  if (WIDE) {
-    const int r = lane & 3, slot = lane >> 2;
-    double acc = 0.0;
-    if (idx < i1) {
-      const int4 rec = orec[idx];
-      i = rec.x;
-      const int n = rec.y;
-      const int64_t p0 = (int64_t)(uint32_t)rec.z | ((int64_t)rec.w << 32);
-#pragma unroll 2
-      for (int s = slot; s < n; s += 4) {
-        const int ck = nbc[p0 + s];
-        const uint64_t pw = pairs[p0 + s];          // asked for together with the colour byte: one memory round trip less on the chain
-        if (LOWER ? ck >= cc : (ck <= cc || ck >= 254)) continue;
-        const int64_t B = (int64_t)(pw & 0xffffffffu);
-        const double4 m = ld256_stream(lu + 16 * (p0 + s) + 4 * r);
-        const double4 zz = ld256(z + B);
-        acc += m.x * zz.x + m.y * zz.y + m.z * zz.z + m.w * zz.w;
-      }
-    }
-    acc += __shfl_down_sync(0xffffffffu, acc, 8, 16);
-    acc += __shfl_down_sync(0xffffffffu, acc, 4, 16);
-    // lanes 0..3 of the group hold the row sums; y = z_i - sums
-    double y = 0.0;
-    if (idx < i1 && slot == 0) y = z[4 * i + r] - acc;
-    if (LOWER) {
-      if (idx < i1 && slot == 0) z[4 * i + r] = y;
-    } else {
-      const double y0 = __shfl_sync(0xffffffffu, y, 0, 16), y1 = __shfl_sync(0xffffffffu, y, 1, 16);
-      const double y2 = __shfl_sync(0xffffffffu, y, 2, 16), y3 = __shfl_sync(0xffffffffu, y, 3, 16);
-      if (idx < i1 && slot == 0) {
-        const double4 d = ld256_nc(dinv + 16 * i + 4 * r);
-        z[4 * i + r] = d.x * y0 + d.y * y1 + d.z * y2 + d.w * y3;
-      }
-    }
-    return;
-  }
-  double acc[4] = {0.0, 0.0, 0.0, 0.0};
-  if (idx < i1) {
-    const int4 rec = orec[idx];
-    i = rec.x;
-    const int n = rec.y;
-    const int64_t p0 = (int64_t)(uint32_t)rec.z | ((int64_t)rec.w << 32);
-    for (int s = lane; s < n; s += 16) {
-      const int ck = nbc[p0 + s];
-      const uint64_t pw = pairs[p0 + s];
-      if (LOWER ? ck >= cc : (ck <= cc || ck >= 254)) continue;
-      const int64_t B = (int64_t)(pw & 0xffffffffu);
-      const double* M = lu + 16 * (p0 + s);
-      const double z0 = z[B], z1 = z[B + 1], z2 = z[B + 2], z3 = z[B + 3];
-#pragma unroll
-      for (int r = 0; r < 4; ++r) acc[r] += M[4 * r] * z0 + M[4 * r + 1] * z1 + M[4 * r + 2] * z2 + M[4 * r + 3] * z3;
-    }
-  }
-#pragma unroll
-  for (int r = 0; r < 4; ++r) {
-#pragma unroll
-    for (int o = 8; o > 0; o >>= 1) acc[r] += __shfl_down_sync(0xffffffffu, acc[r], o, 16);
-  }
-  if (idx < i1 && lane == 0) {
-    double y[4];
-#pragma unroll
-    for (int r = 0; r < 4; ++r) y[r] = z[4 * i + r] - acc[r];
-    if (LOWER) {
-#pragma unroll
-      for (int r = 0; r < 4; ++r) z[4 * i + r] = y[r];
-    } else {
-      const double* D = dinv + 16 * i;
-#pragma unroll
-      for (int r = 0; r < 4; ++r) z[4 * i + r] = D[4 * r] * y[0] + D[4 * r + 1] * y[1] + D[4 * r + 2] * y[2] + D[4 * r + 3] * y[3];
-    }
-  }
-}
-
 // ---- packed factor: counts, fill, refill, sweeps
-__global__ void k_ilu_ecount(int64_t nv, const int4* __restrict__ orec, const uint8_t* __restrict__ nbc, const int32_t* __restrict__ colour,
-                             int64_t* __restrict__ cnt) {
+// per position of the order: the number of owned neighbours of its vertex (its packed blocks)
+__global__ void k_ilu_ecount(int64_t nv, int64_t n_owned, const int32_t* __restrict__ order, const int64_t* __restrict__ pair0,
+                             const int32_t* __restrict__ ns, const uint64_t* __restrict__ pairs, int64_t* __restrict__ cnt) {
   const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (idx > nv) return;
   if (idx == nv) { cnt[idx] = 0; return; }
-  const int4 rec = orec[idx];
-  const int64_t p0 = (int64_t)(uint32_t)rec.z | ((int64_t)rec.w << 32);
+  const int64_t i = order[idx], p0 = pair0[i];
   int m = 0;
-  for (int s = 0; s < rec.y; ++s) m += nbc[p0 + s] < 254 ? 1 : 0;      // 254: the vertex itself, 255: another rank's vertex
+  for (int s = 0; s < ns[i]; ++s) {
+    const int64_t B = (int64_t)(pairs[p0 + s] & 0xffffffffu);
+    m += B < n_owned && (B >> 2) != i ? 1 : 0;
+  }
   cnt[idx] = m;
 }
-__global__ void k_ilu_efill(int64_t nv, const int4* __restrict__ orec, const uint8_t* __restrict__ nbc, const int32_t* __restrict__ colour,
-                            const uint64_t* __restrict__ pairs, const int64_t* __restrict__ eoff, int4* __restrict__ erec, uint32_t* __restrict__ emap,
-                            uint32_t* __restrict__ ecol) {
+// per position of the order: its L blocks (lower colour), then its U blocks, each in neighbour-list order
+__global__ void k_ilu_efill(int64_t nv, int64_t n_owned, const int32_t* __restrict__ order, const int32_t* __restrict__ colour,
+                            const int64_t* __restrict__ pair0, const int32_t* __restrict__ ns, const uint64_t* __restrict__ pairs,
+                            const int64_t* __restrict__ eoff, int4* __restrict__ erec, uint32_t* __restrict__ emap, uint32_t* __restrict__ ecol) {
   const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (idx >= nv) return;
-  const int4 rec = orec[idx];
-  const int64_t p0 = (int64_t)(uint32_t)rec.z | ((int64_t)rec.w << 32);
-  const int cc = colour[rec.x];
+  const int64_t i = order[idx], p0 = pair0[i];
+  const int n = ns[i], cc = colour[i];
   const int64_t q0 = eoff[idx];
   int64_t q = q0;
   int nL = 0, nU = 0;
   for (int pass = 0; pass < 2; ++pass)
-    for (int s = 0; s < rec.y; ++s) {
-      const int ck = nbc[p0 + s];
-      if (ck >= 254 || (pass == 0 ? ck >= cc : ck <= cc)) continue;
+    for (int s = 0; s < n; ++s) {
+      const int64_t B = (int64_t)(pairs[p0 + s] & 0xffffffffu);
+      if (B >= n_owned || (B >> 2) == i) continue;
+      const int ck = colour[B >> 2];
+      if (pass == 0 ? ck >= cc : ck <= cc) continue;
       emap[q] = (uint32_t)(p0 + s);
-      ecol[q] = (uint32_t)(pairs[p0 + s] & 0xffffffffu);
+      ecol[q] = (uint32_t)B;
       ++q;
       if (pass == 0) ++nL; else ++nU;
     }
-  erec[idx] = make_int4(rec.x, nL | (nU << 16), (int)(q0 & 0xffffffffLL), (int)(q0 >> 32));
+  erec[idx] = make_int4((int)i, nL | (nU << 16), (int)(q0 & 0xffffffffLL), (int)(q0 >> 32));
 }
 // packed blocks <- factor (four lanes per block, one 32-byte row each)
 __global__ void k_ilu_pack(int64_t n_packed, const uint32_t* __restrict__ emap, const double* __restrict__ lu, double* __restrict__ lue) {
@@ -546,7 +396,7 @@ k_ilu_sweep_packed(int64_t i0, int64_t i1, const int4* __restrict__ erec, const 
 void ilu_free(nsgpu_ctx* ctx) {
   IluPlan* P = static_cast<IluPlan*>(ctx->ilu);
   if (!P) return;
-  cudaFree(P->d_colour); cudaFree(P->d_order); cudaFree(P->d_lu); cudaFree(P->d_dinv); cudaFree(P->d_nbc); cudaFree(P->d_orec);
+  cudaFree(P->d_colour); cudaFree(P->d_order); cudaFree(P->d_lu); cudaFree(P->d_dinv);
   cudaFree(P->d_erec); cudaFree(P->d_emap); cudaFree(P->d_ecol); cudaFree(P->d_lue);
   delete P;
   ctx->ilu = nullptr;
@@ -554,118 +404,72 @@ void ilu_free(nsgpu_ctx* ctx) {
 
 static inline unsigned g256(int64_t n) { return (unsigned)ceil_div(n > 0 ? n : 1, 256); }
 
-// colouring and elimination order (once per pattern)
+// colouring, elimination order and the packed layout of the factor (once per pattern)
 static int ilu_plan(nsgpu_ctx* ctx, const P1BlockView& V) {
   ilu_free(ctx);
-  IluPlan* P = new IluPlan();
-  ctx->ilu = P;
   cudaStream_t s = ctx->stream;
   const int64_t nv = ctx->n_owned / 4;
+  if (ctx->n_owned % 4 != 0 || nv <= 0 || nv > V.n_ent || nv >= (int64_t(1) << 31)) {
+    set_error(ctx, "pc = 5: the owned rows are not whole vertices, or more than 2^31 vertices");
+    return NSGPU_EUNSUPPORTED;
+  }
+  if (ctx->n_pairs >= (int64_t(1) << 32)) { set_error(ctx, "pc = 5: 2^32 or more neighbour blocks on one rank"); return NSGPU_EUNSUPPORTED; }
+  IluPlan* P = new IluPlan();
+  ctx->ilu = P;
   P->nv = nv;
   int* d_flag = nullptr;
-  unsigned long long* d_cnt = nullptr;
-  uint64_t *d_keys = nullptr, *d_keys2 = nullptr;
+  int64_t *d_ecnt = nullptr, *d_eoff = nullptr;
   void* d_tmp = nullptr;
-  auto cleanup = [&]() { cudaFree(d_flag); cudaFree(d_cnt); cudaFree(d_keys); cudaFree(d_keys2); cudaFree(d_tmp); };
+  auto done = [&](int rc, const std::string& msg) {   // msg empty: the callee has set the message
+    if (!msg.empty()) set_error(ctx, msg);
+    cudaFree(d_flag); cudaFree(d_ecnt); cudaFree(d_eoff); cudaFree(d_tmp);
+    if (rc) ilu_free(ctx);
+    return rc;
+  };
 #define IL_CUDA(call)                                                                              \
   do {                                                                                             \
     cudaError_t e__ = (call);                                                                      \
-    if (e__ != cudaSuccess) {                                                                      \
-      set_error(ctx, std::string("ilu: " #call ": ") + cudaGetErrorString(e__));                   \
-      cleanup(); ilu_free(ctx);                                                                    \
-      return NSGPU_ECUDA;                                                                          \
-    }                                                                                              \
+    if (e__ != cudaSuccess) return done(NSGPU_ECUDA, std::string("pc = 5: " #call ": ") + cudaGetErrorString(e__)); \
   } while (0)
   IL_CUDA(cudaMalloc(&d_flag, 2 * sizeof(int)));
-  IL_CUDA(cudaMalloc(&d_cnt, 65 * sizeof(unsigned long long)));
   IL_CUDA(cudaMemsetAsync(d_flag, 0, 2 * sizeof(int), s));
-  if (ctx->n_owned % 4 != 0 || nv <= 0 || nv > V.n_ent || nv >= (int64_t(1) << 31)) { P->unsupported = true; cleanup(); return NSGPU_OK; }
   k_ilu_check<<<g256(nv), 256, 0, s>>>(nv, V.rowdof, d_flag);
-  int rc;
-  if ((rc = dev_alloc(ctx, &P->d_colour, nv)) || (rc = dev_alloc(ctx, &P->d_order, nv))) { cleanup(); ilu_free(ctx); return rc; }
-  IL_CUDA(cudaMemsetAsync(P->d_colour, 0xff, sizeof(int32_t) * nv, s));
-  int32_t* d_prev = reinterpret_cast<int32_t*>(P->d_order);   // round-start snapshot (the order array is filled later)
-  for (int round = 0; round < 1000; ++round) {
-    IL_CUDA(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), s));
-    IL_CUDA(cudaMemcpyAsync(d_prev, P->d_colour, sizeof(int32_t) * nv, cudaMemcpyDeviceToDevice, s));
-    k_ilu_colour<<<g256(nv), 256, 0, s>>>(nv, ctx->n_owned, V.pair0, V.ns, ctx->d_pairs, d_prev, P->d_colour, d_cnt, d_flag + 1);
-    unsigned long long left = 0;
-    IL_CUDA(cudaMemcpyAsync(&left, d_cnt, sizeof(left), cudaMemcpyDeviceToHost, s));
-    IL_CUDA(cudaStreamSynchronize(s));
-    ctx->launches += 1;
-    if (left == 0) break;
-  }
+  k_ilu_maxns<<<g256(nv), 256, 0, s>>>(nv, V.ns, d_flag + 1);
   int flags[2] = {0, 0};
   IL_CUDA(cudaMemcpyAsync(flags, d_flag, sizeof(flags), cudaMemcpyDeviceToHost, s));
   IL_CUDA(cudaStreamSynchronize(s));
-  if (flags[0] || flags[1]) { P->unsupported = true; cleanup(); return NSGPU_OK; }   // not the blocked numbering / more than 64 colours
-  IL_CUDA(cudaMalloc(&d_keys, sizeof(uint64_t) * nv));
-  IL_CUDA(cudaMalloc(&d_keys2, sizeof(uint64_t) * nv));
-  k_ilu_keys<<<g256(nv), 256, 0, s>>>(nv, P->d_colour, d_keys);
-  size_t tmp_bytes = 0;
-  IL_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, d_keys, d_keys2, nv, 0, 40, s));
-  IL_CUDA(cudaMalloc(&d_tmp, tmp_bytes));
-  IL_CUDA(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_keys, d_keys2, nv, 0, 40, s));
-  IL_CUDA(cudaMemsetAsync(d_cnt, 0, 65 * sizeof(unsigned long long), s));
-  k_ilu_order<<<g256(nv), 256, 0, s>>>(nv, d_keys2, P->d_order, d_cnt);
-  unsigned long long cnt[65];
-  IL_CUDA(cudaMemcpyAsync(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, s));
-  IL_CUDA(cudaStreamSynchronize(s));
-  IL_CUDA(cudaGetLastError());
-  ctx->launches += 3;
-  P->cstart.assign(1, 0);
-  for (int c = 0; c < 64; ++c) {
-    if (cnt[c] == 0) break;
-    P->cstart.push_back(P->cstart.back() + (int64_t)cnt[c]);
-  }
-  P->n_colours = (int)P->cstart.size() - 1;
-  if (P->cstart.back() != nv) { P->unsupported = true; cleanup(); return NSGPU_OK; }
-  if ((rc = dev_alloc(ctx, &P->d_lu, 16 * ctx->n_pairs)) || (rc = dev_alloc(ctx, &P->d_dinv, 16 * nv)) || (rc = dev_alloc(ctx, &P->d_nbc, ctx->n_pairs)) ||
-      (rc = dev_alloc(ctx, &P->d_orec, nv))) {
-    cleanup(); ilu_free(ctx); return rc;
-  }
-  k_ilu_nbc<<<g256(nv * 16), 256, 0, s>>>(nv, ctx->n_owned, V.pair0, V.ns, ctx->d_pairs, P->d_colour, P->d_nbc);
-  k_ilu_orec<<<g256(nv), 256, 0, s>>>(nv, P->d_order, V.pair0, V.ns, P->d_orec);
   ctx->launches += 2;
-  IL_CUDA(cudaGetLastError());
-  IL_CUDA(cudaMemsetAsync(d_flag, 0, sizeof(int), s));
-  k_ilu_maxns<<<g256(nv), 256, 0, s>>>(nv, V.ns, d_flag);
-  IL_CUDA(cudaMemcpyAsync(&P->max_ns, d_flag, sizeof(int), cudaMemcpyDeviceToHost, s));
+  if (flags[0]) return done(NSGPU_EUNSUPPORTED, "pc = 5: the numbering is not vertex-blocked");
+  P->max_ns = flags[1];
+  IL_CUDA(cudaMalloc(&P->d_colour, sizeof(int32_t) * nv));
+  IL_CUDA(cudaMalloc(&P->d_order, sizeof(int32_t) * nv));
+  // vertex e's rows are 4e .. 4e + 3, and row 4e holds the dofs of exactly its neighbour vertices
+  if (int rc = mc_colour(ctx, nv, 2, nullptr, 64, "pc = 5", P->d_colour, P->d_order, P->cstart, nullptr)) return done(rc, "");
+  P->n_colours = (int)P->cstart.size() - 1;
+  IL_CUDA(cudaMalloc(&P->d_lu, sizeof(double) * 16 * ctx->n_pairs));
+  IL_CUDA(cudaMalloc(&P->d_dinv, sizeof(double) * 16 * nv));
+  IL_CUDA(cudaMalloc(&P->d_erec, sizeof(int4) * nv));
+  IL_CUDA(cudaMalloc(&d_ecnt, sizeof(int64_t) * (nv + 1)));
+  IL_CUDA(cudaMalloc(&d_eoff, sizeof(int64_t) * (nv + 1)));
+  k_ilu_ecount<<<g256(nv + 1), 256, 0, s>>>(nv, ctx->n_owned, P->d_order, V.pair0, V.ns, ctx->d_pairs, d_ecnt);
+  size_t tb = 0;
+  IL_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb, d_ecnt, d_eoff, nv + 1, s));
+  IL_CUDA(cudaMalloc(&d_tmp, tb));
+  IL_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tb, d_ecnt, d_eoff, nv + 1, s));
+  int64_t np = 0;
+  IL_CUDA(cudaMemcpyAsync(&np, d_eoff + nv, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
   IL_CUDA(cudaStreamSynchronize(s));
-  ctx->launches += 1;
-  // packed factor tables (optional: without the memory for a second copy of the blocks the sweeps walk d_lu through the neighbour lists)
-  if (ctx->ilu_packed) {
-    int64_t *d_ecnt = nullptr, *d_eoff = nullptr;
-    void* d_tmp2 = nullptr;
-    bool ok = cudaMalloc(&d_ecnt, sizeof(int64_t) * (nv + 1)) == cudaSuccess && cudaMalloc(&d_eoff, sizeof(int64_t) * (nv + 1)) == cudaSuccess;
-    if (ok) {
-      k_ilu_ecount<<<g256(nv + 1), 256, 0, s>>>(nv, P->d_orec, P->d_nbc, P->d_colour, d_ecnt);
-      size_t tb = 0;
-      ok = cub::DeviceScan::ExclusiveSum(nullptr, tb, d_ecnt, d_eoff, nv + 1, s) == cudaSuccess && cudaMalloc(&d_tmp2, tb) == cudaSuccess &&
-           cub::DeviceScan::ExclusiveSum(d_tmp2, tb, d_ecnt, d_eoff, nv + 1, s) == cudaSuccess;
-    }
-    int64_t np = 0;
-    if (ok) ok = cudaMemcpyAsync(&np, d_eoff + nv, sizeof(int64_t), cudaMemcpyDeviceToHost, s) == cudaSuccess && cudaStreamSynchronize(s) == cudaSuccess;
-    if (ok && np > 0 && np < (int64_t(1) << 32) && ctx->n_pairs < (int64_t(1) << 32)) {
-      ok = cudaMalloc(&P->d_erec, sizeof(int4) * nv) == cudaSuccess && cudaMalloc(&P->d_emap, sizeof(uint32_t) * np) == cudaSuccess &&
-           cudaMalloc(&P->d_ecol, sizeof(uint32_t) * np) == cudaSuccess && cudaMalloc(&P->d_lue, sizeof(double) * 16 * np) == cudaSuccess;
-      if (ok) {
-        k_ilu_efill<<<g256(nv), 256, 0, s>>>(nv, P->d_orec, P->d_nbc, P->d_colour, ctx->d_pairs, d_eoff, P->d_erec, P->d_emap, P->d_ecol);
-        ok = cudaStreamSynchronize(s) == cudaSuccess && cudaGetLastError() == cudaSuccess;
-        ctx->launches += 2;
-        P->n_packed = np;
-      }
-    } else ok = false;
-    if (!ok) {   // not fatal: fall back to the unpacked sweeps
-      cudaGetLastError();
-      cudaFree(P->d_erec); cudaFree(P->d_emap); cudaFree(P->d_ecol); cudaFree(P->d_lue);
-      P->d_erec = nullptr; P->d_emap = nullptr; P->d_ecol = nullptr; P->d_lue = nullptr; P->n_packed = 0;
-    }
-    cudaFree(d_ecnt); cudaFree(d_eoff); cudaFree(d_tmp2);
-  }
-  cleanup();
+  if (np >= (int64_t(1) << 32)) return done(NSGPU_EUNSUPPORTED, "pc = 5: 2^32 or more packed factor blocks on one rank");
+  P->n_packed = np;
+  IL_CUDA(cudaMalloc(&P->d_emap, sizeof(uint32_t) * (np > 0 ? np : 1)));
+  IL_CUDA(cudaMalloc(&P->d_ecol, sizeof(uint32_t) * (np > 0 ? np : 1)));
+  IL_CUDA(cudaMalloc(&P->d_lue, sizeof(double) * 16 * (np > 0 ? np : 1)));
+  k_ilu_efill<<<g256(nv), 256, 0, s>>>(nv, ctx->n_owned, P->d_order, P->d_colour, V.pair0, V.ns, ctx->d_pairs, d_eoff, P->d_erec, P->d_emap, P->d_ecol);
+  ctx->launches += 3;
+  IL_CUDA(cudaStreamSynchronize(s));
+  IL_CUDA(cudaGetLastError());
 #undef IL_CUDA
-  return NSGPU_OK;
+  return done(NSGPU_OK, "");
 }
 
 // factorise the Jacobian now resident in ctx->d_vals.  NSGPU_EUNSUPPORTED when the vertex-blocked view does not exist.
@@ -678,7 +482,6 @@ int ilu_factor(nsgpu_ctx* ctx) {
     if (rc) return rc;
     P = static_cast<IluPlan*>(ctx->ilu);
   }
-  if (P->unsupported) { set_error(ctx, "pc = ILU: the numbering is not vertex-blocked or the vertex graph needs more than 64 colours"); return NSGPU_EUNSUPPORTED; }
   cudaStream_t s = ctx->stream;
   int* d_sing = nullptr;
   NS_CUDA(ctx, cudaMalloc(&d_sing, sizeof(int)));
@@ -686,18 +489,15 @@ int ilu_factor(nsgpu_ctx* ctx) {
   k_ilu_load<<<g256(P->nv * 16), 256, 0, s>>>(P->nv, ctx->n_owned, V.pair0, V.ns, ctx->d_pairs, V.rowpos, ctx->d_vals, P->d_lu);
   for (int c = 0; c < P->n_colours; ++c) {
     const int64_t i0 = P->cstart[c], i1 = P->cstart[c + 1];
-    if (P->max_ns <= 16 && ctx->ilu_factor16)
+    if (P->max_ns <= 16)
       k_ilu_factor16<<<(unsigned)ceil_div(i1 - i0, 8), 128, 0, s>>>(i0, i1, c, ctx->n_owned, P->d_order, P->d_colour, V.pair0, V.ns, ctx->d_pairs, P->d_lu,
                                                                       P->d_dinv, d_sing);
     else
       k_ilu_factor<<<(unsigned)ceil_div(i1 - i0, 64), 64, 0, s>>>(i0, i1, c, ctx->n_owned, P->d_order, P->d_colour, V.pair0, V.ns, ctx->d_pairs, P->d_lu,
                                                                      P->d_dinv, d_sing);
   }
-  ctx->launches += 1 + P->n_colours;
-  if (P->d_lue) {
-    k_ilu_pack<<<g256(P->n_packed * 4), 256, 0, s>>>(P->n_packed, P->d_emap, P->d_lu, P->d_lue);
-    ctx->launches += 1;
-  }
+  k_ilu_pack<<<g256(P->n_packed * 4), 256, 0, s>>>(P->n_packed, P->d_emap, P->d_lu, P->d_lue);
+  ctx->launches += 2 + P->n_colours;
   int sing = 0;
   cudaError_t e = cudaMemcpyAsync(&sing, d_sing, sizeof(int), cudaMemcpyDeviceToHost, s);
   if (e == cudaSuccess) e = cudaStreamSynchronize(s);
@@ -708,36 +508,23 @@ int ilu_factor(nsgpu_ctx* ctx) {
   return NSGPU_OK;
 }
 
-// d_z (owned entries) = U^-1 L^-1 d_r.  d_z may alias d_r.
+// d_z (owned entries) = U^-1 L^-1 d_r.  d_z may alias d_r and must be 32-byte aligned (256-bit loads).
 int ilu_apply(nsgpu_ctx* ctx, const double* d_r, double* d_z) {
   IluPlan* P = static_cast<IluPlan*>(ctx->ilu);
-  P1BlockView V;
-  if (!P || P->unsupported || !P->d_lu || !p1tet_block_view(ctx, &V)) { set_error(ctx, "ilu_apply: no factorisation"); return NSGPU_EINVAL; }
+  if (!P) { set_error(ctx, "ilu_apply: no factorisation"); return NSGPU_EINVAL; }
+  if (((reinterpret_cast<uintptr_t>(d_z) | reinterpret_cast<uintptr_t>(P->d_lue)) & 31) != 0) {
+    set_error(ctx, "ilu_apply: the vector and the factor must be 32-byte aligned");
+    return NSGPU_EINVAL;
+  }
   cudaStream_t s = ctx->stream;
   if (d_z != d_r) NS_CUDA(ctx, cudaMemcpyAsync(d_z, d_r, sizeof(double) * (size_t)ctx->n_owned, cudaMemcpyDeviceToDevice, s));
-  const bool wide = (reinterpret_cast<uintptr_t>(d_z) & 31) == 0 && (reinterpret_cast<uintptr_t>(P->d_lu) & 31) == 0;   // 256-bit loads
-  if (wide && P->d_lue) {
-    for (int c = 1; c < P->n_colours; ++c) {
-      const int64_t i0 = P->cstart[c], i1 = P->cstart[c + 1];
-      k_ilu_sweep_packed<true><<<g256((i1 - i0) * 16), 256, 0, s>>>(i0, i1, P->d_erec, P->d_ecol, P->d_lue, P->d_dinv, d_z);
-    }
-    for (int c = P->n_colours - 1; c >= 0; --c) {
-      const int64_t i0 = P->cstart[c], i1 = P->cstart[c + 1];
-      k_ilu_sweep_packed<false><<<g256((i1 - i0) * 16), 256, 0, s>>>(i0, i1, P->d_erec, P->d_ecol, P->d_lue, P->d_dinv, d_z);
-    }
-    ctx->launches += 2 * P->n_colours - 1;
-    NS_CUDA(ctx, cudaGetLastError());
-    return NSGPU_OK;
-  }
   for (int c = 1; c < P->n_colours; ++c) {
     const int64_t i0 = P->cstart[c], i1 = P->cstart[c + 1];
-    if (wide) k_ilu_sweep<true, true><<<g256((i1 - i0) * 16), 256, 0, s>>>(i0, i1, c, P->d_orec, P->d_nbc, ctx->d_pairs, P->d_lu, P->d_dinv, d_z);
-    else k_ilu_sweep<true, false><<<g256((i1 - i0) * 16), 256, 0, s>>>(i0, i1, c, P->d_orec, P->d_nbc, ctx->d_pairs, P->d_lu, P->d_dinv, d_z);
+    k_ilu_sweep_packed<true><<<g256((i1 - i0) * 16), 256, 0, s>>>(i0, i1, P->d_erec, P->d_ecol, P->d_lue, P->d_dinv, d_z);
   }
   for (int c = P->n_colours - 1; c >= 0; --c) {
     const int64_t i0 = P->cstart[c], i1 = P->cstart[c + 1];
-    if (wide) k_ilu_sweep<false, true><<<g256((i1 - i0) * 16), 256, 0, s>>>(i0, i1, c, P->d_orec, P->d_nbc, ctx->d_pairs, P->d_lu, P->d_dinv, d_z);
-    else k_ilu_sweep<false, false><<<g256((i1 - i0) * 16), 256, 0, s>>>(i0, i1, c, P->d_orec, P->d_nbc, ctx->d_pairs, P->d_lu, P->d_dinv, d_z);
+    k_ilu_sweep_packed<false><<<g256((i1 - i0) * 16), 256, 0, s>>>(i0, i1, P->d_erec, P->d_ecol, P->d_lue, P->d_dinv, d_z);
   }
   ctx->launches += 2 * P->n_colours - 1;
   NS_CUDA(ctx, cudaGetLastError());
@@ -746,7 +533,7 @@ int ilu_apply(nsgpu_ctx* ctx, const double* d_r, double* d_z) {
 
 int ilu_colours(nsgpu_ctx* ctx, int32_t* h_colour, int32_t* n_colours) {
   IluPlan* P = static_cast<IluPlan*>(ctx->ilu);
-  if (!P || P->unsupported || !P->d_colour) { set_error(ctx, "ilu_colours: no factorisation"); return NSGPU_EINVAL; }
+  if (!P) { set_error(ctx, "ilu_colours: no factorisation"); return NSGPU_EINVAL; }
   if (n_colours) *n_colours = P->n_colours;
   if (h_colour) {
     NS_CUDA(ctx, cudaMemcpyAsync(h_colour, P->d_colour, sizeof(int32_t) * (size_t)P->nv, cudaMemcpyDeviceToHost, ctx->stream));

@@ -738,11 +738,6 @@ int nsgpu_set_option(nsgpu_ctx* ctx, const char* name, int64_t value) {
   } else if (!strcmp(name, "rowown")) {
     NS_REQUIRE(ctx, value >= 0 && value <= 2, "set_option: rowown must be 0 (never), 1 (P2-P1 spaces) or 2 (every space without a factorised kernel)");
     ctx->rowown = (int)value;
-  } else if (!strcmp(name, "ilu_factor16")) {
-    ctx->ilu_factor16 = value != 0;
-  } else if (!strcmp(name, "ilu_packed")) {
-    ctx->ilu_packed = value != 0;
-    ilu_free(ctx);
   } else if (!strcmp(name, "spmv_wide")) {
     ctx->spmv_wide = value != 0;
   } else if (!strcmp(name, "rowown_lean")) {

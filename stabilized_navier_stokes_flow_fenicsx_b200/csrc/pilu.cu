@@ -6,11 +6,11 @@
 // 4x4-block variant that needs the vertex-blocked P1-P1 tet layout).  Columns of other ranks are dropped: block Jacobi over ranks.
 //
 //   classes     a dof is pressure when it sits at a cell-local position >= gdim * (velocity nodes per cell) of the dofmap
-//   colouring   Jones-Plassmann with hashed priorities and round-start snapshots (deterministic) on the owned graph of the CSR
-//               pattern: the velocity dofs first, then the pressure dofs with colours numbered after every velocity colour.  Every
-//               pressure row is therefore eliminated after all its velocity neighbours and its pivot picks up the local Schur term
-//               -sum B A^-1 B^T; with one colouring over all dofs a zero pressure diagonal (Taylor-Hood Stokes, beta = 0) comes first
-//               and the factorisation breaks down.
+//   colouring   Jones-Plassmann with hashed priorities and round-start snapshots (deterministic; colour.cu, shared with pc = 5) on the
+//               owned graph of the CSR pattern: the velocity dofs first, then the pressure dofs with colours numbered after every
+//               velocity colour, at most PILU_MAX_COLOURS in all.  Every pressure row is therefore eliminated after all its velocity
+//               neighbours and its pivot picks up the local Schur term -sum B A^-1 B^T; with one colouring over all dofs a zero
+//               pressure diagonal (Taylor-Hood Stokes, beta = 0) comes first and the factorisation breaks down.
 //   order       elimination order = (colour, row); rows of one colour share no matrix entry
 //   factorise   one launch per colour, one warp per row (IKJ variant, Saad alg. 10.4): for every earlier neighbour k in elimination
 //               order  a_ik /= u_kk ;  a_ij -= a_ik u_kj  for every later j of row i's pattern with (k, j) in the pattern
@@ -25,7 +25,6 @@
 namespace nsgpu {
 
 constexpr int PILU_MAX_COLOURS = 2048;   // velocity + pressure colours (the P2 velocity graph needs tens of them)
-constexpr int PILU_MAX_ROUNDS = 1000;    // Jones-Plassmann rounds per class
 
 struct PiluPlan {
   int64_t n = 0;                    // owned rows
@@ -45,11 +44,6 @@ struct PiluPlan {
   bool factored = false;            // d_lue / d_uinv hold a usable factorisation of the current values
 };
 
-__device__ __forceinline__ uint32_t pilu_hash(uint32_t x) {
-  x ^= x >> 16; x *= 0x7feb352du; x ^= x >> 15; x *= 0x846ca68bu; x ^= x >> 16;
-  return x;
-}
-
 // pressure flag per owned row from the cell-local position of the dof
 __global__ void k_pilu_classify(int64_t n_cells, int nd, int first_p, int64_t n_owned, const int32_t* __restrict__ dofmap, uint8_t* isp) {
   const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -59,55 +53,14 @@ __global__ void k_pilu_classify(int64_t n_cells, int nd, int first_p, int64_t n_
   if (d >= 0 && d < n_owned) isp[d] = 1;
 }
 
-// one Jones-Plassmann round over the rows of class cls: an uncoloured row whose priority beats every uncoloured neighbour of its
-// class takes the lowest colour >= base that no neighbour of its class holds.  Decisions use the colours at the start of the round.
-__global__ void k_pilu_colour(int64_t n, const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices, const uint8_t* __restrict__ isp,
-                              int cls, int base, const int32_t* __restrict__ colour, int32_t* colour_out, unsigned long long* state) {
-  const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (e >= n || isp[e] != cls || colour[e] >= 0) return;
-  const uint32_t pe = pilu_hash((uint32_t)e);
-  const int64_t b = indptr[e], end = indptr[e + 1];
-  for (int64_t p = b; p < end; ++p) {
-    const int64_t j = indices[p];
-    if (j >= n || j == e || isp[j] != cls || colour[j] >= 0) continue;
-    const uint32_t pj = pilu_hash((uint32_t)j);
-    if (pj > pe || (pj == pe && j > e)) { atomicAdd(state, 1ull); return; }   // a neighbour goes first
-  }
-  for (int w = base; w < PILU_MAX_COLOURS; w += 64) {
-    unsigned long long used = 0;
-    for (int64_t p = b; p < end; ++p) {
-      const int64_t j = indices[p];
-      if (j >= n || j == e || isp[j] != cls) continue;
-      const int cj = colour[j];
-      if (cj >= w && cj < w + 64) used |= 1ull << (cj - w);
-    }
-    if (~used) {
-      const int c = w + __ffsll((long long)~used) - 1;
-      if (c < PILU_MAX_COLOURS) { colour_out[e] = c; return; }
-      break;
-    }
-  }
-  state[1] = 1ull;   // colour limit: the row stays uncoloured and the plan is refused
-}
-
-__global__ void k_pilu_maxc(int64_t n, const int32_t* __restrict__ colour, int* out) {
-  const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (e < n) atomicMax(out, colour[e]);
-}
-
-__global__ void k_pilu_keys(int64_t n, const int32_t* __restrict__ colour, uint64_t* keys) {
-  const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (e < n) keys[e] = ((uint64_t)(uint32_t)colour[e] << 32) | (uint64_t)e;
-}
-
 // per position of the elimination order: its row and the sizes of its L (earlier colour) and U (later colour) parts
-__global__ void k_pilu_count(int64_t n, const uint64_t* __restrict__ keys, const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices,
-                             const int32_t* __restrict__ colour, int4* erec, int64_t* cnt, unsigned long long* ccount) {
+__global__ void k_pilu_count(int64_t n, const int32_t* __restrict__ order, const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices,
+                             const int32_t* __restrict__ colour, int4* erec, int64_t* cnt) {
   const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (idx > n) return;
   if (idx == n) { cnt[idx] = 0; return; }
-  const int64_t i = (int64_t)(keys[idx] & 0xffffffffu);
-  const int c = (int)(keys[idx] >> 32);
+  const int64_t i = order[idx];
+  const int c = colour[i];
   int nL = 0, nU = 0;
   for (int64_t p = indptr[i]; p < indptr[i + 1]; ++p) {
     const int64_t j = indices[p];
@@ -116,7 +69,6 @@ __global__ void k_pilu_count(int64_t n, const uint64_t* __restrict__ keys, const
   }
   erec[idx] = make_int4((int)i, nL | (nU << 16), 0, 0);
   cnt[idx] = nL + nU;
-  atomicAdd(ccount + c, 1ull);
 }
 
 // packed entries of each position in CSR order, keyed by (colour of the column, column): sorted per row, the L part comes first
@@ -240,91 +192,47 @@ static int pilu_plan(nsgpu_ctx* ctx) {
   ctx->pilu = P;
   P->n = n;
   uint8_t* d_isp = nullptr;
-  int32_t* d_prev = nullptr;
-  unsigned long long* d_state = nullptr;
-  uint64_t *d_keys = nullptr, *d_keys2 = nullptr, *d_ekey = nullptr, *d_ekey2 = nullptr;
+  int32_t* d_order = nullptr;
+  uint64_t *d_ekey = nullptr, *d_ekey2 = nullptr;
   int64_t *d_cnt = nullptr, *d_eoff = nullptr, *d_epos = nullptr;
-  int* d_max = nullptr;
   void* d_tmp = nullptr;
-  auto cleanup = [&]() {
-    cudaFree(d_isp); cudaFree(d_prev); cudaFree(d_state); cudaFree(d_keys); cudaFree(d_keys2); cudaFree(d_ekey); cudaFree(d_ekey2);
-    cudaFree(d_cnt); cudaFree(d_eoff); cudaFree(d_epos); cudaFree(d_max); cudaFree(d_tmp);
-  };
-  auto fail = [&](int rc, const std::string& msg) {
-    set_error(ctx, msg);
-    cleanup(); pilu_free(ctx);
+  auto done = [&](int rc, const std::string& msg) {   // msg empty: the callee has set the message
+    if (!msg.empty()) set_error(ctx, msg);
+    cudaFree(d_isp); cudaFree(d_order); cudaFree(d_ekey); cudaFree(d_ekey2); cudaFree(d_cnt); cudaFree(d_eoff); cudaFree(d_epos); cudaFree(d_tmp);
+    if (rc) pilu_free(ctx);
     return rc;
   };
 #define PL_CUDA(call)                                                                              \
   do {                                                                                             \
     cudaError_t e__ = (call);                                                                      \
-    if (e__ != cudaSuccess) return fail(NSGPU_ECUDA, std::string("pc = 6: " #call ": ") + cudaGetErrorString(e__)); \
+    if (e__ != cudaSuccess) return done(NSGPU_ECUDA, std::string("pc = 6: " #call ": ") + cudaGetErrorString(e__)); \
   } while (0)
   PL_CUDA(cudaMalloc(&d_isp, n));
-  PL_CUDA(cudaMalloc(&d_prev, sizeof(int32_t) * n));
-  PL_CUDA(cudaMalloc(&d_state, 2 * sizeof(unsigned long long) + PILU_MAX_COLOURS * sizeof(unsigned long long)));
-  PL_CUDA(cudaMalloc(&d_max, sizeof(int)));
+  PL_CUDA(cudaMalloc(&d_order, sizeof(int32_t) * n));
   PL_CUDA(cudaMalloc(&P->d_colour, sizeof(int32_t) * n));
   PL_CUDA(cudaMemsetAsync(d_isp, 0, n, s));
-  PL_CUDA(cudaMemsetAsync(P->d_colour, 0xff, sizeof(int32_t) * n, s));
   const int first_p = ctx->gdim * ctx->nent;
   k_pilu_classify<<<pg256(ctx->n_cells_total * (ctx->nd - first_p)), 256, 0, s>>>(ctx->n_cells_total, ctx->nd, first_p, n, ctx->d_dofmap, d_isp);
   ctx->launches += 1;
   // velocity rows (class 0) from colour 0, then pressure rows (class 1) from the first colour after the velocity ones
-  int base = 0;
-  for (int cls = 0; cls < 2; ++cls) {
-    unsigned long long st[2] = {1, 0};
-    int round = 0;
-    for (; round < PILU_MAX_ROUNDS && st[0] != 0; ++round) {
-      PL_CUDA(cudaMemsetAsync(d_state, 0, 2 * sizeof(unsigned long long), s));
-      PL_CUDA(cudaMemcpyAsync(d_prev, P->d_colour, sizeof(int32_t) * n, cudaMemcpyDeviceToDevice, s));
-      k_pilu_colour<<<pg256(n), 256, 0, s>>>(n, ctx->d_indptr, ctx->d_indices, d_isp, cls, base, d_prev, P->d_colour, d_state);
-      PL_CUDA(cudaMemcpyAsync(st, d_state, sizeof(st), cudaMemcpyDeviceToHost, s));
-      PL_CUDA(cudaStreamSynchronize(s));
-      ctx->launches += 1;
-      if (st[1]) return fail(NSGPU_EUNSUPPORTED, "pc = 6: the matrix graph needs more than " + std::to_string(PILU_MAX_COLOURS) + " colours");
-    }
-    if (st[0] != 0) return fail(NSGPU_EUNSUPPORTED, "pc = 6: the colouring did not finish in " + std::to_string(PILU_MAX_ROUNDS) + " rounds");
-    PL_CUDA(cudaMemsetAsync(d_max, 0xff, sizeof(int), s));
-    k_pilu_maxc<<<pg256(n), 256, 0, s>>>(n, P->d_colour, d_max);
-    int mx = -1;
-    PL_CUDA(cudaMemcpyAsync(&mx, d_max, sizeof(int), cudaMemcpyDeviceToHost, s));
-    PL_CUDA(cudaStreamSynchronize(s));
-    ctx->launches += 1;
-    if (cls == 0) P->n_vel_colours = mx + 1;
-    base = mx + 1;
-  }
-  P->n_colours = base;
-  // elimination order (colour, row), per-colour counts and the packed layout
-  PL_CUDA(cudaMalloc(&d_keys, sizeof(uint64_t) * n));
-  PL_CUDA(cudaMalloc(&d_keys2, sizeof(uint64_t) * n));
-  k_pilu_keys<<<pg256(n), 256, 0, s>>>(n, P->d_colour, d_keys);
-  size_t tb = 0;
-  PL_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, tb, d_keys, d_keys2, n, 0, 44, s));
-  PL_CUDA(cudaMalloc(&d_tmp, tb));
-  PL_CUDA(cub::DeviceRadixSort::SortKeys(d_tmp, tb, d_keys, d_keys2, n, 0, 44, s));
-  cudaFree(d_tmp); d_tmp = nullptr;
+  if (int rc = mc_colour(ctx, n, 0, d_isp, PILU_MAX_COLOURS, "pc = 6", P->d_colour, d_order, P->cstart, &P->n_vel_colours)) return done(rc, "");
+  P->n_colours = (int)P->cstart.size() - 1;
+  // the packed layout
   PL_CUDA(cudaMalloc(&P->d_erec, sizeof(int4) * n));
   PL_CUDA(cudaMalloc(&d_cnt, sizeof(int64_t) * (n + 1)));
   PL_CUDA(cudaMalloc(&d_eoff, sizeof(int64_t) * (n + 1)));
-  unsigned long long* d_ccount = d_state + 2;
-  PL_CUDA(cudaMemsetAsync(d_ccount, 0, PILU_MAX_COLOURS * sizeof(unsigned long long), s));
-  k_pilu_count<<<pg256(n + 1), 256, 0, s>>>(n, d_keys2, ctx->d_indptr, ctx->d_indices, P->d_colour, P->d_erec, d_cnt, d_ccount);
+  k_pilu_count<<<pg256(n + 1), 256, 0, s>>>(n, d_order, ctx->d_indptr, ctx->d_indices, P->d_colour, P->d_erec, d_cnt);
+  size_t tb = 0;
   PL_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb, d_cnt, d_eoff, n + 1, s));
   PL_CUDA(cudaMalloc(&d_tmp, tb));
   PL_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tb, d_cnt, d_eoff, n + 1, s));
   cudaFree(d_tmp); d_tmp = nullptr;
-  std::vector<unsigned long long> ccount(P->n_colours);
   int64_t np = 0;
-  PL_CUDA(cudaMemcpyAsync(ccount.data(), d_ccount, sizeof(unsigned long long) * P->n_colours, cudaMemcpyDeviceToHost, s));
   PL_CUDA(cudaMemcpyAsync(&np, d_eoff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
   PL_CUDA(cudaMemcpyAsync(&P->nnz_owned, ctx->d_indptr + n, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
   PL_CUDA(cudaStreamSynchronize(s));
-  ctx->launches += 4;
-  P->cstart.assign(1, 0);
-  for (int c = 0; c < P->n_colours; ++c) P->cstart.push_back(P->cstart.back() + (int64_t)ccount[c]);
-  if (P->cstart.back() != n) return fail(NSGPU_EUNSUPPORTED, "pc = 6: inconsistent colouring");
-  if (np >= (int64_t(1) << 31)) return fail(NSGPU_EUNSUPPORTED, "pc = 6: more than 2^31 owned off-diagonal entries on one rank");
+  ctx->launches += 2;
+  if (np >= (int64_t(1) << 31)) return done(NSGPU_EUNSUPPORTED, "pc = 6: more than 2^31 owned off-diagonal entries on one rank");
   P->n_packed = np;
   PL_CUDA(cudaMalloc(&d_ekey, sizeof(uint64_t) * (np > 0 ? np : 1)));
   PL_CUDA(cudaMalloc(&d_ekey2, sizeof(uint64_t) * (np > 0 ? np : 1)));
@@ -350,9 +258,8 @@ static int pilu_plan(nsgpu_ctx* ctx) {
   // lanes per row of the sweeps from the mean length of a row's L or U part (the CSR SpMV's rule on whole rows)
   const double avg = (double)np / (double)n;
   P->lpr = avg > 48 ? 16 : (avg > 24 ? 8 : 4);
-  cleanup();
 #undef PL_CUDA
-  return NSGPU_OK;
+  return done(NSGPU_OK, "");
 }
 
 // factorise the matrix now resident in ctx->d_vals.  NSGPU_EZEROPIVOT (on every rank) when a pivot is zero or not finite.

@@ -1,11 +1,13 @@
-"""Multicolour block ILU(0) preconditioner of the device-resident TFQMR (csrc/ilu.cu, pc = 5): the factorisation against a NumPy
-restatement of block ILU(0) in the same elimination order (oracle/ilu_ref.py), and the solve against a sparse LU."""
+"""Multicolour block ILU(0) preconditioner of the device-resident TFQMR (csrc/ilu.cu, pc = 5): the colouring against its NumPy
+restatement (oracle/colour_ref.py), the factorisation against a NumPy restatement of block ILU(0) in the same elimination order
+(oracle/ilu_ref.py), and the solve against a sparse LU."""
 import numpy as np
 import pytest
 import scipy.sparse as sps
 import scipy.sparse.linalg as spla
+from scipy.spatial import Delaunay
 
-from oracle import ilu_ref
+from oracle import colour_ref, ilu_ref
 from stabilized_navier_stokes_flow_fenicsx_b200 import mesh as M
 from stabilized_navier_stokes_flow_fenicsx_b200.assembler import NSAssembler
 
@@ -33,6 +35,7 @@ def test_ilu_application_matches_the_block_ilu0_restatement():
     G = sps.coo_matrix((np.ones(A.nnz), (A.tocoo().row // 4, A.tocoo().col // 4))).tocsr().tocoo()
     off = G.row != G.col
     assert np.all(colour[G.row[off]] != colour[G.col[off]])
+    assert np.array_equal(colour, colour_ref.colour(indptr, indices, sp.n_dofs // 4, shift=2))
     blocks, dinv, order, rank = ilu_ref.block_ilu0(indptr, indices, vals, colour)
     zr = ilu_ref.apply(blocks, dinv, order, rank, r)
     assert np.abs(z - zr).max() <= 1e-10 * np.abs(zr).max()
@@ -42,13 +45,42 @@ def test_ilu_application_matches_the_block_ilu0_restatement():
     assert e_ilu < 0.9
     z2 = asm.ilu_apply(r)                       # same colouring, same factors: bitwise reproducible
     assert np.array_equal(z, z2)
-    asm.set_option("ilu_factor16", 0)           # one thread per vertex instead of sixteen lanes: the same operations per block
-    z4 = asm.ilu_apply(r)
-    assert np.abs(z4 - z).max() <= 1e-13 * np.abs(z).max()
-    asm.set_option("ilu_factor16", 1)
-    asm.set_option("ilu_packed", 0)             # sweeps through the neighbour lists instead of the packed copy of the factor
-    z3 = asm.ilu_apply(r)
-    assert np.abs(z3 - zr).max() <= 1e-10 * np.abs(zr).max() and np.abs(z3 - z).max() <= 1e-12 * np.abs(z).max()
+    asm.close()
+
+
+def _delaunay_setup():
+    """P1-P1 on a Delaunay tetrahedralisation of a 7x7x7 lattice with jittered interior points, velocity fixed on the boundary: block
+    rows longer than 16, which the sixteen-lane factorisation kernel does not take."""
+    g = np.linspace(0.0, 1.0, 7)
+    x = np.stack(np.meshgrid(g, g, g, indexing="ij"), -1).reshape(-1, 3)
+    inner = np.all((x > 0) & (x < 1), axis=1)
+    x[inner] += np.random.default_rng(2).uniform(-0.04, 0.04, (inner.sum(), 3))
+    tets = Delaunay(x).simplices
+    p = x[tets]
+    vol = np.abs(np.einsum("ij,ij->i", np.cross(p[:, 1] - p[:, 0], p[:, 2] - p[:, 0]), p[:, 3] - p[:, 0]))
+    m = M.Mesh(3, x, np.ascontiguousarray(tets[vol > 1e-12], dtype=np.int32))     # drop the flat slivers on the faces of the cube
+    sp = M.mixed_space(m, 1)
+    bnd = np.flatnonzero(np.any((sp.dof_x == 0.0) | (sp.dof_x == 1.0), axis=1) & (sp.dof_comp < 3)).astype(np.int32)
+    asm = NSAssembler(m.x, m.cells, sp.dofmap, vdeg=1, options={"renumber": 0})
+    asm.set_form(flavour=0, nu=0.1); asm.set_bcs([(bnd, np.zeros(len(bnd)))])
+    indptr, indices = asm.create_matrix()
+    w = 0.1 * np.random.default_rng(4).standard_normal(sp.n_dofs)
+    w[bnd] = 0.0
+    vals = asm.jacobian(w)
+    return sp, asm, indptr, indices, vals
+
+
+def test_ilu_application_with_block_rows_longer_than_16():
+    sp, asm, indptr, indices, vals = _delaunay_setup()
+    assert (np.diff(indptr)[::4] // 4).max() > 16          # blocks in the longest block row
+    r = np.random.default_rng(3).standard_normal(sp.n_dofs)
+    z = asm.ilu_apply(r)
+    colour, nc = asm.ilu_colours()
+    assert np.array_equal(colour, colour_ref.colour(indptr, indices, sp.n_dofs // 4, shift=2))
+    blocks, dinv, order, rank = ilu_ref.block_ilu0(indptr, indices, vals, colour)
+    zr = ilu_ref.apply(blocks, dinv, order, rank, r)
+    assert np.abs(z - zr).max() <= 1e-10 * np.abs(zr).max()
+    assert np.array_equal(z, asm.ilu_apply(r))
     asm.close()
 
 

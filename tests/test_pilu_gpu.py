@@ -11,7 +11,7 @@ import scipy.sparse as sps
 import scipy.sparse.linalg as spla
 
 import _pins as P
-from oracle import pilu_ref
+from oracle import colour_ref, pilu_ref
 from stabilized_navier_stokes_flow_fenicsx_b200 import mesh as M
 from stabilized_navier_stokes_flow_fenicsx_b200._lib import NsgpuError
 from stabilized_navier_stokes_flow_fenicsx_b200.assembler import NSAssembler
@@ -28,7 +28,7 @@ def _dirichlet_state(n, bcs):
     return w
 
 
-def _case(name):
+def _case(name, options=None):
     """(assembler, CSR pattern + values in the caller's numbering, right-hand side, pressure flag per dof) of a Newton-step system."""
     if name == "cavity_ugn_p1":
         m = M.create_rectangle_tris(24, 24); sp = M.mixed_space(m, 1)
@@ -51,7 +51,7 @@ def _case(name):
         w = np.empty(sp.n_dofs); w[perm] = M.duct_state(sp)
         is_p = np.empty(sp.n_dofs, dtype=bool); is_p[perm] = sp.dof_comp == 3
         fk = dict(flavour=0, nu=0.1)
-    asm = NSAssembler(m.x, m.cells, dofmap, vdeg=sp.vdeg)
+    asm = NSAssembler(m.x, m.cells, dofmap, vdeg=sp.vdeg, options=options)
     asm.set_form(**fk); asm.set_bcs(bcs)
     indptr, indices = asm.create_matrix()
     vals, F = asm.jacobian_residual(w)
@@ -77,6 +77,16 @@ def test_pilu_application_matches_the_ilu0_restatement(name):
     assert np.abs(z - zr).max() <= 1e-10 * np.abs(zr).max(), np.abs(z - zr).max() / np.abs(zr).max()
     assert np.array_equal(z, asm.pilu_apply(r))                       # same colouring, same factor: bitwise reproducible
     assert np.array_equal(z, asm.pilu_apply(r, refactor=False))
+    asm.close()
+
+
+@pytest.mark.parametrize("name", CASES[:3])
+def test_pilu_colours_match_the_colouring_restatement(name):
+    asm, indptr, indices, vals, F, is_p = _case(name, options={"renumber": 0})     # internal numbering = the caller's
+    colour, nc, nvc = asm.pilu_colours()
+    ref = colour_ref.colour(indptr, indices, asm.n_owned, cls=is_p)
+    assert np.array_equal(colour, ref)
+    assert nc == ref.max() + 1 and nvc == ref[~is_p].max() + 1
     asm.close()
 
 

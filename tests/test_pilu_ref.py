@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 import _pins as P
-from oracle import pilu_ref
+from oracle import colour_ref, pilu_ref
 from stabilized_navier_stokes_flow_fenicsx_b200 import mesh as M
 
 
@@ -74,3 +74,17 @@ def test_pilu_ref_pressure_first_meets_a_zero_pivot(oracle):
     colour = greedy_colouring(indptr, indices, is_p, pressure_first=True)
     with pytest.raises(ZeroDivisionError, match="zero pivot"):
         pilu_ref.pilu0(indptr, indices, vals, colour)
+
+
+def test_colour_ref_is_a_proper_colouring_velocity_first(oracle):
+    """The colouring restatement (oracle/colour_ref.py) that tests/test_ilu_gpu.py and tests/test_pilu_gpu.py hold the device colours
+    to: no two neighbours share a colour, and every pressure colour comes after every velocity colour."""
+    for name, sp, (indptr, indices, vals) in _cases(oracle):
+        n = sp.n_dofs
+        is_p = sp.dof_comp == sp.mesh.gdim
+        colour = colour_ref.colour(indptr, indices, n, cls=is_p)
+        rows = np.repeat(np.arange(n), np.diff(indptr))
+        off = rows != indices
+        assert colour.min() == 0 and np.all(colour[rows[off]] != colour[indices[off]]), name
+        assert colour[~is_p].max() + 1 == colour[is_p].min(), name
+        assert np.array_equal(np.unique(colour), np.arange(colour.max() + 1)), name
