@@ -204,9 +204,11 @@ NS_HD void p1tet_rowslab(const FormParams& fp, const bool row_is_origin, const d
 //       A_vv[c][d] = C0[c][d] + [n == 0] e^2 W D[c][d] + L Q[c][d] + uq_n[c] t1[d] + g_0[c] t2[d] + delta_cd dia
 //       A_pv[d]    = P0[d] + W g_n[d] + t1[d] + s[d] L
 //     with t1 = e W tau_n (H - tau_n^2 a_0(n) Gu_n),  t2 = e W tau_n kappa Gu_n + nuL g_n   (per block: ~70 FMA);
-//   * the per-point data of points 1..3 is parked by `scratch` (the kernel uses the thread's own, not yet written,
-//     staging slots in shared memory) and fetched back right before the block that needs it;
-//   * each finished 4x4 block is handed to `emit(n, blk)` immediately (Dirichlet handling + staging store).
+//   * the per-point data of points 1..3 is parked by `scratch` (the warp-specialised kernel uses the thread's lane of
+//     tensor memory, the other kernels its own, not yet written, staging slots in shared memory) and fetched back right
+//     before the block that needs it;
+//   * each finished 4x4 block is handed to `emit(n, blk)` immediately (Dirichlet handling + staging store), the first one
+//     after `scratch.before_first_emit()`.
 // Live state during the block loop is ~55 doubles instead of ~100, which gives ptxas room to interleave the
 // independent FMA chains (the fp64 pipe needs ILP >= 2 at 8 warps/SM: tools/microbench.cu).
 struct P1TetPoint { double uq[3], Gu[3], ew, eb, ea; };   // ew = e W tau, eb = e W tau^3 a_0, ea = e W tau a_0
@@ -270,7 +272,7 @@ NS_HD void p1tet_rowslab2(const FormParams& fp, const bool row_is_origin, const 
   for (int d = 0; d < 3; ++d) H[d] = D[d][0] * g[0][0] + D[d][1] * g[0][1] + D[d][2] * g[0][2];
   const double Pg0 = P[0] * g[0][0] + P[1] * g[0][1] + P[2] * g[0][2];
   // the point loop needs neither grad u nor the gradients of the other three vertices: the caller may take them out of the
-  // register file until the block loop (shared-memory scratch in the kernels; a plain copy on the host)
+  // register file until the block loop (tensor-memory or shared-memory scratch in the kernels)
   scratch.put_geom(g, D);
 
   // ---- quadrature points: totals stay in registers, the data of points 1..3 is parked ----
@@ -382,6 +384,9 @@ NS_HD void p1tet_rowslab2(const FormParams& fp, const bool row_is_origin, const 
 #pragma unroll
       for (int d = 0; d < 3; ++d) blk[12 + d] = P0[d] + W * g[n][d] + t1[d] + s[d] * L;
       blk[15] = tbar * L;
+      // a scratch kept outside the caller's output area lets the caller wait for that area only here; no lane-divergent branch
+      // in this function encloses the block loop, so every thread of a warp that runs it reaches this point
+      if (n == 0) scratch.before_first_emit();
       emit(n, blk);
     }
   }

@@ -405,6 +405,7 @@ template <int CAP, int ECAP = CAP> struct TileSmem {
 
 template <int CAP_, bool WANT_J, int ECAP = CAP_> struct TileView {
   static constexpr int CAP = CAP_;
+  static constexpr bool tmem_scratch = false;   // phase-A scratch in the thread's own staging slots (no tensor memory allocated)
   double2* stageJ; double4* stageF; int64_t* rowpos; int4* rowdof; int2* rel; uint32_t* src; uint8_t* bytes;
   __device__ explicit TileView(unsigned char* raw) {
     stageJ = reinterpret_cast<double2*>(raw);
@@ -588,9 +589,56 @@ __device__ __forceinline__ void tile_gather(const View& v, const TileHdr& h, int
 
 struct NoHook { __device__ __forceinline__ void operator()() const {} };
 
+// Tensor-memory transfers of the 32x32b shape (sm_100a): lane i of the warp reaches lane (lane base of `a`) + i, and a double
+// occupies two consecutive 32-bit columns (lo, hi).  A transfer of 2N columns starts at a column that is a multiple of 2N.
+// Loads include the tcgen05.wait::ld, so their values are complete when the function returns.
+#define NS_TM_LH(v) "r"(__double2loint(v)), "r"(__double2hiint(v))
+__device__ __forceinline__ void tmem_st1(uint32_t a, double x0) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};" ::"r"(a), NS_TM_LH(x0) : "memory");
+}
+__device__ __forceinline__ void tmem_st2(uint32_t a, double x0, double x1) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(a), NS_TM_LH(x0), NS_TM_LH(x1) : "memory");
+}
+__device__ __forceinline__ void tmem_st8(uint32_t a, const double (&x)[8]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(a),
+               NS_TM_LH(x[0]), NS_TM_LH(x[1]), NS_TM_LH(x[2]), NS_TM_LH(x[3]), NS_TM_LH(x[4]), NS_TM_LH(x[5]), NS_TM_LH(x[6]), NS_TM_LH(x[7])
+               : "memory");
+}
+__device__ __forceinline__ void tmem_st16(uint32_t a, const double (&x)[16]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+               "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};" ::"r"(a),
+               NS_TM_LH(x[0]), NS_TM_LH(x[1]), NS_TM_LH(x[2]), NS_TM_LH(x[3]), NS_TM_LH(x[4]), NS_TM_LH(x[5]), NS_TM_LH(x[6]), NS_TM_LH(x[7]),
+               NS_TM_LH(x[8]), NS_TM_LH(x[9]), NS_TM_LH(x[10]), NS_TM_LH(x[11]), NS_TM_LH(x[12]), NS_TM_LH(x[13]), NS_TM_LH(x[14]), NS_TM_LH(x[15])
+               : "memory");
+}
+#undef NS_TM_LH
+__device__ __forceinline__ void tmem_ld1(uint32_t a, double& x0) {
+  uint32_t r[2];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];\n\ttcgen05.wait::ld.sync.aligned;" : "=r"(r[0]), "=r"(r[1]) : "r"(a) : "memory");
+  x0 = __hiloint2double(r[1], r[0]);
+}
+__device__ __forceinline__ void tmem_ld2(uint32_t a, double& x0, double& x1) {
+  uint32_t r[4];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n\ttcgen05.wait::ld.sync.aligned;"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(a) : "memory");
+  x0 = __hiloint2double(r[1], r[0]); x1 = __hiloint2double(r[3], r[2]);
+}
+__device__ __forceinline__ void tmem_ld8(uint32_t a, double (&x)[8]) {
+  uint32_t r[16];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n\t"
+               "tcgen05.wait::ld.sync.aligned;"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
+                 "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+               : "r"(a) : "memory");
+#pragma unroll
+  for (int i = 0; i < 8; ++i) x[i] = __hiloint2double(r[2 * i + 1], r[2 * i]);
+}
+
 // `before_first_write` is called exactly once, by every thread that runs the function, before anything is written into the
-// tile view (staging area): the pipelined kernel places there the barrier that waits for the previous tile's gather, so
-// that the geometry / first quadrature point of the next tile overlap the tail of that gather.
+// tile view (staging area): the pipelined and the warp-specialised kernels place there the barrier that waits for the gather
+// of the tile that used the view before, so that the start of this tile's algebra overlaps the tail of that gather.  Where
+// the scratch lives in the staging slots (SmemScratch) that is right after the geometry, when grad u is parked; where it
+// lives in tensor memory (TmemScratch) it is right before the first block is emitted, after the whole point loop.
 template <int CAP, bool WANT_J, bool WANT_F, class View, class Hook = NoHook>
 __device__ __forceinline__ void phase_a_core(const View& v, const int tid, const int (&lead)[4], const uint32_t cm, const double (&x)[4][3],
                                              const double (&u)[4][3], const double (&p)[4], P1_PHASE_ARGS, Hook before_first_write = Hook()) {
@@ -635,7 +683,48 @@ __device__ __forceinline__ void phase_a_core(const View& v, const int tid, const
         }
       }
     };
-    if (WANT_J) {
+    if constexpr (WANT_J && View::tmem_scratch) {
+      // Scratch in the thread's tensor-memory lane.  Columns counted from the compute group's first one (a double = a lo/hi pair):
+      //   0..35                grad u (D[0][0] .. D[2][2]), then the gradients of vertices 1..3
+      //   32 + 16 q .. 47 + 16 q  uq, Gu, ew, eb of point q = 1..3;   94 + 2 q, 95 + 2 q  its ea
+      // Nothing is parked in the staging buffer, which is therefore needed only from the first emitted block on.
+      struct TmemScratch {
+        uint32_t a;
+        Hook& hook;
+        __device__ double after_geometry(double w) const { return w; }
+        __device__ void put_geom(const double (&g)[4][3], const double (&D)[3][3]) const {
+          const double x[16] = {D[0][0], D[0][1], D[0][2], D[1][0], D[1][1], D[1][2], D[2][0], D[2][1],
+                                D[2][2], g[1][0], g[1][1], g[1][2], g[2][0], g[2][1], g[2][2], g[3][0]};
+          tmem_st16(a, x);
+          tmem_st2(a + 32, g[3][1], g[3][2]);
+        }
+        __device__ void get_D(double (&D)[3][3]) const {
+          asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");   // every put precedes get_D: all later loads see the parked values
+          double x[8];
+          tmem_ld8(a, x);
+          D[0][0] = x[0]; D[0][1] = x[1]; D[0][2] = x[2]; D[1][0] = x[3]; D[1][1] = x[4]; D[1][2] = x[5]; D[2][0] = x[6]; D[2][1] = x[7];
+          tmem_ld1(a + 16, D[2][2]);
+        }
+        __device__ void get_g(int n, double (&gn)[3]) const {
+          const uint32_t c = a + 18 + 6 * (n - 1);   // 18, 24, 30: split so that each transfer starts on a multiple of its width
+          if (n & 1) { tmem_ld1(c, gn[0]); tmem_ld2(c + 2, gn[1], gn[2]); }
+          else { tmem_ld2(c, gn[0], gn[1]); tmem_ld1(c + 4, gn[2]); }
+        }
+        __device__ void put(int q, const P1TetPoint& pt) const {
+          const double x[8] = {pt.uq[0], pt.uq[1], pt.uq[2], pt.Gu[0], pt.Gu[1], pt.Gu[2], pt.ew, pt.eb};
+          tmem_st8(a + 32 + 16 * q, x);
+          tmem_st1(a + 94 + 2 * q, pt.ea);
+        }
+        __device__ void get(int q, P1TetPoint& pt) const {
+          double x[8];
+          tmem_ld8(a + 32 + 16 * q, x);
+          pt.uq[0] = x[0]; pt.uq[1] = x[1]; pt.uq[2] = x[2]; pt.Gu[0] = x[3]; pt.Gu[1] = x[4]; pt.Gu[2] = x[5]; pt.ew = x[6]; pt.eb = x[7];
+          tmem_ld1(a + 94 + 2 * q, pt.ea);
+        }
+        __device__ void before_first_emit() const { hook(); }   // first write into the view
+      } scratch{v.tmem, before_first_write};
+      p1tet_rowslab2<true, WANT_F>(form, row_is_origin, x, u, p, fr, scratch, emit);
+    } else if constexpr (WANT_J) {
       // point data of q = 1..3 waits in the (not yet written) staging slot of block q
       struct SmemScratch {
         double2* st;   // staging area; the five pieces of point q wait in pieces 0..4 of the thread's (not yet written) block q
@@ -647,43 +736,29 @@ __device__ __forceinline__ void phase_a_core(const View& v, const int tid, const
         // forwarding the stored registers to the loads
         __device__ void put_geom(const double (&g)[4][3], const double (&D)[3][3]) const {
           hook();   // first write into the view
-#ifndef NS_NO_PARK
           sts2(stage_idx(CAP, 0, 0, tid), D[0][0], D[0][1]); sts2(stage_idx(CAP, 0, 1, tid), D[0][2], D[1][0]);
           sts2(stage_idx(CAP, 0, 2, tid), D[1][1], D[1][2]); sts2(stage_idx(CAP, 0, 3, tid), D[2][0], D[2][1]);
-#ifndef NS_PARK_D_ONLY
           sts2(stage_idx(CAP, 0, 4, tid), D[2][2], g[1][2]); sts2(stage_idx(CAP, 0, 5, tid), g[2][2], g[3][2]);
 #pragma unroll
           for (int n = 1; n < 4; ++n) sts2(stage_idx(CAP, n, 5, tid), g[n][0], g[n][1]);
-#else
-          sts2(stage_idx(CAP, 0, 4, tid), D[2][2], 0.0);
-          (void)g;
-#endif
-#endif
         }
         __device__ void get_D(double (&D)[3][3]) const {
-#ifndef NS_NO_PARK
           double t;
           lds2(stage_idx(CAP, 0, 0, tid), D[0][0], D[0][1]); lds2(stage_idx(CAP, 0, 1, tid), D[0][2], D[1][0]);
           lds2(stage_idx(CAP, 0, 2, tid), D[1][1], D[1][2]); lds2(stage_idx(CAP, 0, 3, tid), D[2][0], D[2][1]);
           lds2(stage_idx(CAP, 0, 4, tid), D[2][2], t);
-#ifndef NS_PARK_D_ONLY
           // the z components of the three parked gradients ride in block 0's pieces 4 and 5, which block 0 overwrites when it is
           // emitted: move them next to the x / y components (piece 6 of their own blocks)
           double g2, g3;
           lds2(stage_idx(CAP, 0, 5, tid), g2, g3);
           sts2(stage_idx(CAP, 1, 6, tid), t, 0.0); sts2(stage_idx(CAP, 2, 6, tid), g2, 0.0); sts2(stage_idx(CAP, 3, 6, tid), g3, 0.0);
-#endif
-#endif
         }
         __device__ void get_g(int n, double (&gn)[3]) const {
-#if !defined(NS_NO_PARK) && !defined(NS_PARK_D_ONLY)
           double pad;
           lds2(stage_idx(CAP, n, 5, tid), gn[0], gn[1]);
           lds2(stage_idx(CAP, n, 6, tid), gn[2], pad);
-#else
-          (void)n; (void)gn;
-#endif
         }
+        __device__ void before_first_emit() const {}   // the hook ran in put_geom
         // 128-bit shared accesses the compiler neither widens, splits nor forwards from registers
         __device__ void sts2(int idx, double a, double b) const {
           asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"((unsigned)__cvta_generic_to_shared(st + idx)), "d"(a), "d"(b) : "memory");
@@ -714,6 +789,7 @@ __device__ __forceinline__ void phase_a_core(const View& v, const int tid, const
         __device__ void get_g(int, double (&)[3]) const {}
         __device__ void put(int i, const P1TetPoint& pt) { q[i] = pt; }
         __device__ void get(int i, P1TetPoint& pt) const { pt = q[i]; }
+        __device__ void before_first_emit() const {}
       } scratch;
       before_first_write();   // ahead of the (lane-divergent) choice below: the barrier it may hold must be reached uniformly
       if (has_bc) p1tet_rowslab2<true, WANT_F>(form, row_is_origin, x, u, p, fr, scratch, emit);

@@ -286,8 +286,21 @@ __device__ __forceinline__ void mbar_wait(uint64_t* b, uint32_t parity) {
   } while (!ok);
 }
 
-// named barriers: FULL[b] = 1 + b, EMPTY[b] = 4 + b (256 threads: one compute group + the gather group), compute group g: 7 + g, gather group: 9
-struct WsView { double2* stageJ; double4* stageF; };
+// tensor memory: 256 columns per CTA, compute group g owns columns [128 g, 128 g + 128) (the phase-A scratch, TmemScratch in
+// p1tet.cu).  One CTA runs per SM (shared memory and the 512 x 128 registers limit residency), so the concurrent launches of the
+// streamed path (p1tet_assemble_streamed, three streams) never hold columns on the same SM at once, and 256 of the 512 columns
+// could not be contended for even if two CTAs were co-resident.
+constexpr int WS_TMEM_COLS = 256;
+__device__ __forceinline__ void tmem_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tmem_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+
+// named barriers: FULL[b] = 1 + b, EMPTY[b] = 4 + b (256 threads: one compute group + the gather group), compute group g: 7 + g, gather group h: 9 + h,
+// end of the kernel: 11 (512 threads)
+// tmem: tensor-memory address of the warp's 32 lanes (32 * (warp % 4)) at the compute group's first column
+struct WsView {
+  static constexpr bool tmem_scratch = true;
+  double2* stageJ; double4* stageF; uint32_t tmem;
+};
 
 // phase B of one tile by the 128 threads of a gather warpgroup (48 registers per thread: plain loops; the two gather
 // groups of a CTA work on alternate tiles, so each SM sub-partition has two gather warps to hide each other's latencies).
@@ -375,12 +388,21 @@ k_p1tet_ws(const FormParams form, const double* __restrict__ xg, const double* _
   const int wg = threadIdx.x >> 7;         // 0, 1: compute warpgroups; 2, 3: gather warpgroups
   const int tid = threadIdx.x & 127;
   const int nk = (int)((n_tiles - (int64_t)blockIdx.x + gridDim.x - 1) / gridDim.x);   // tiles of this CTA: tile0 + blockIdx.x + k * gridDim.x
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + S::off_bar);                   // TAB[3], RING[2][2]
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + S::off_bar);                   // TAB[3], RING[2][2], tensor-memory address
+  // the slot that holds the tensor-memory address, as a 32-bit shared address (a constant: nothing to keep live across the roles)
+  const uint32_t tmem_slot = smem_u32(smem_raw) + (uint32_t)(S::off_bar + 7 * sizeof(uint64_t));
+  auto tmem_base = [&]() { uint32_t a; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(a) : "r"(tmem_slot) : "memory"); return a; };
+  // allocated in every instantiation, also the residual-only <false, true> one whose register scratch never touches it: one
+  // lifecycle for all three keeps the barrier and the deallocation below identical on every path, and costs one allocation per CTA
+  if (threadIdx.x < 32)
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "n"(WS_TMEM_COLS) : "memory");
   if (threadIdx.x == 0) {
     for (int i = 0; i < 7; ++i) mbar_init(bars + i, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
+  tmem_fence_before();
   __syncthreads();
+  tmem_fence_after();
   auto stage_of = [&](int b) { return smem_raw + (size_t)b * S::stage; };
   if (wg < 2) {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(WS_REG_COMPUTE));
@@ -437,7 +459,8 @@ k_p1tet_ws(const FormParams form, const double* __restrict__ xg, const double* _
       }
       cp_async_commit();
       if (tid == 0 && m + 2 < nm) fetch_ring(m + 2);
-      const WsView v{reinterpret_cast<double2*>(stage_of(b)), reinterpret_cast<double4*>(stage_of(b) + (WANT_J ? (size_t)32 * WS_SS * sizeof(double2) : 0))};
+      const WsView v{reinterpret_cast<double2*>(stage_of(b)), reinterpret_cast<double4*>(stage_of(b) + (WANT_J ? (size_t)32 * WS_SS * sizeof(double2) : 0)),
+                     tmem_base() + ((uint32_t)(tid & 96) << 16) + 128u * g};
       auto wait_empty = [&]() { if (k >= WS_NBUF) named_bar_sync(4 + b, 256); };   // the gather group is done with tile k - 3
       const int col = tid < WS_SS ? tid : tid - 8;
       if ((tid & ~31) < ninc)
@@ -447,8 +470,18 @@ k_p1tet_ws(const FormParams form, const double* __restrict__ xg, const double* _
       __threadfence_block();
       named_bar_arrive(1 + b, 256);          // FULL[b]
     }
+    // end of the kernel (also with nk == 0): every thread of the CTA takes part in barrier 11 (the gather groups arrive as they
+    // start), and the tensor memory goes back once both compute groups have made their last access
+    tmem_fence_before();
+    named_bar_sync(11, 512);
+    if (threadIdx.x < 32) {
+      tmem_fence_after();
+      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base()), "n"(WS_TMEM_COLS) : "memory");
+      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
   } else {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(WS_REG_GATHER));
+    named_bar_arrive(11, 512);               // end-of-kernel barrier: the gather groups never access tensor memory
     // ---------------------------------------------------------------- gather warpgroup h: tiles j = h, h + 2, ... (parked by compute group h)
     const int h = wg - 2;
     unsigned char* htab = smem_raw + S::off_htab;
