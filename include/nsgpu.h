@@ -247,7 +247,7 @@ int nsgpu_get_rows(nsgpu_ctx* ctx, int64_t n, const int32_t* rows, int64_t* star
  * One GPU thread integrates one seed with scipy's RK45 algorithm (solve_ivp(..., method='RK45', events=..., max_step=...)),
  * locating the point in the tetrahedral mesh of nsgpu_set_mesh and evaluating the P1 velocity there; zero outside the mesh.
  *
- * nsgpu_trace_setup  builds the point locator (first call / new tol) and loads the nodal velocity u_nodes (n_nodes x 3, the
+ * nsgpu_trace_setup  builds the mesh's point locator (first use; shared with nsgpu_eval) and loads the nodal velocity u_nodes (n_nodes x 3, the
  *                    geometry-node order of nsgpu_set_mesh; NULL keeps the previous field).  Replaces geometry.bb_tree(mesh, 3)
  *                    (streamtrace.py:397) and the Function uh filled by read_mesh_and_function (:57-129).  tol: a point is inside
  *                    a cell when every barycentric coordinate is >= -tol.
@@ -262,6 +262,38 @@ int nsgpu_trace_velocity(nsgpu_ctx* ctx, int64_t n, const double* points, double
 int nsgpu_trace_run(nsgpu_ctx* ctx, int64_t n, const double* seeds, int reverse, double x_stop, double speed_min, double t_end,
                     double max_step, double rtol, double atol, int64_t max_steps, double* end_xyz, int32_t* status, double* t_final,
                     int32_t* n_steps);
+
+/* ---- point evaluation and non-matching interpolation of the mixed function (Function.eval / Function.interpolate_nonmatching:
+ *      NavierStokesChannelFlow.py:150-157 inlet profiles, :175-194 interpolate_initial_guess of the coarse w onto the fine W;
+ *      DFG_2D_Validation.py's uh.eval of the pressure at two points) ------------------------------------------------------------
+ * Point location uses the context's locator (per-cell affine maps + a uniform bin grid with sorted per-bin cell lists, built on
+ * first use of the mesh and shared with the streamline tracer).  Rule for a point p:
+ *   1. inside: the lowest-numbered cell of p's bin whose barycentric coordinates are all >= -tol;
+ *   2. extrapolation, only when step 1 finds no cell and padding > 0: among the cells of the bins the box [p - padding, p + padding]
+ *      overlaps, the one at the smallest Euclidean distance from p to the closed cell (ties to the lower cell number), accepted when
+ *      that distance is <= padding; that cell's polynomials are evaluated at p;
+ *   3. otherwise outside: the values are 0.
+ * Single rank only: both contexts must have one rank (NSGPU_EUNSUPPORTED otherwise; distributed point ownership, dolfinx's
+ * determine_point_ownership, is not implemented).  NSGPU_EINVAL for NULL arrays, a negative tol or padding, a context without
+ * mesh and space, differing gdim or contexts on different devices; nothing is changed then.
+ *
+ * nsgpu_eval: w_local (n_owned + n_ghost values, caller numbering) at n points (n x 3; z ignored on triangles).  values: n x (gdim+1),
+ *   the velocity components then the pressure.  cell (may be NULL): c when the point is inside cell c, -2 - c when extrapolated
+ *   from cell c, -1 outside.  P1 or P2 velocity, P1 pressure, triangles or tetrahedra.
+ * nsgpu_interpolate: called with the destination: every dof of w_dst (n_owned + n_ghost of dst, caller numbering) is set to the
+ *   source function w_src evaluated at the dof's node (vertices; edge midpoints 0.5 (xa + xb) for P2), each node located once.
+ *   The meshes may differ in resolution, cell order, numbering and velocity degree (P1-P1 -> P2-P1 is allowed); gdim must agree.
+ *   n_extrapolated / n_outside (may be NULL): destination nodes that took step 2 / step 3.
+ * The _dev variants take device pointers (the counts too) and are asynchronous on the stream of ctx / dst; dst's stream first waits
+ * for the work queued on src's.  The first call on a mesh builds its locator (synchronous). */
+int nsgpu_eval(nsgpu_ctx* ctx, const double* w_local, int64_t n, const double* points, double tol, double padding, double* values,
+               int32_t* cell);
+int nsgpu_eval_dev(nsgpu_ctx* ctx, const double* w_local_dev, int64_t n, const double* points_dev, double tol, double padding,
+                   double* values_dev, int32_t* cell_dev);
+int nsgpu_interpolate(nsgpu_ctx* src, const double* w_src, nsgpu_ctx* dst, double* w_dst, double tol, double padding,
+                      int64_t* n_extrapolated, int64_t* n_outside);
+int nsgpu_interpolate_dev(nsgpu_ctx* src, const double* w_src_dev, nsgpu_ctx* dst, double* w_dst_dev, double tol, double padding,
+                          int64_t* n_extrapolated_dev, int64_t* n_outside_dev);
 
 #ifdef __cplusplus
 }

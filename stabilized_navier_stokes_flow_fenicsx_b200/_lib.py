@@ -84,6 +84,10 @@ SIGNATURES = {
     "nsgpu_trace_setup": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.c_double]),
     "nsgpu_trace_velocity": (ctypes.c_int, [c_ctx, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "nsgpu_trace_run": (ctypes.c_int, [c_ctx, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int] + [ctypes.c_double] * 6 + [ctypes.c_int64] + [ctypes.c_void_p] * 4),
+    "nsgpu_eval": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
+    "nsgpu_eval_dev": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
+    "nsgpu_interpolate": (ctypes.c_int, [c_ctx, ctypes.c_void_p, c_ctx, ctypes.c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
+    "nsgpu_interpolate_dev": (ctypes.c_int, [c_ctx, ctypes.c_void_p, c_ctx, ctypes.c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
 }
 
 

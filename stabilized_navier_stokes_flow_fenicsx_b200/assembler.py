@@ -335,6 +335,45 @@ class NSAssembler:
                 self.dev_free(Jd_dev)
         return hist
 
+    # ------------------------------------------------------------------ point evaluation / non-matching interpolation
+    def eval(self, w, points, tol=1e-12, padding=0.0):
+        """Function.eval of the mixed function w (caller numbering) at points (n, 3): returns (values (n, gdim + 1) = velocity
+        components then pressure, cells (n,) int32).  cells: c inside cell c (lowest-numbered cell with every barycentric coordinate
+        >= -tol), -2 - c extrapolated from the nearest cell c within ``padding``, -1 outside (values 0).  One rank only."""
+        w = self._state(w)
+        p = np.ascontiguousarray(points, dtype=np.float64)
+        if p.ndim != 2 or p.shape[1] != 3:
+            raise ValueError("points must be (n, 3)")
+        values = np.empty((p.shape[0], self.gdim + 1))
+        cells = np.empty(p.shape[0], dtype=np.int32)
+        self._check(self.lib.nsgpu_eval(self.ctx, _ptr(w), p.shape[0], _ptr(p), float(tol), float(padding), _ptr(values), _ptr(cells)), "eval")
+        return values, cells
+
+    def eval_dev(self, w_dev, n, points_dev, values_dev, cells_dev=None, tol=1e-12, padding=0.0):
+        """``eval`` on device arrays (w: n_owned + n_ghost, points: n x 3, values: n x (gdim + 1) doubles, cells: n int32 or None);
+        asynchronous on the context's stream."""
+        self._check(self.lib.nsgpu_eval_dev(self.ctx, w_dev, int(n), points_dev, float(tol), float(padding), values_dev, cells_dev), "eval_dev")
+
+    def interpolate_nonmatching(self, src, w_src, tol=1e-12, padding=0.0):
+        """Function.interpolate_nonmatching onto this (destination) space: every dof gets the source function ``w_src`` of the
+        NSAssembler ``src`` (another mesh of the same gdim, any velocity degree) evaluated at the dof's node, with the location rule
+        of ``eval``.  Returns (w (n_owned + n_ghost), info = dict(n_extrapolated, n_outside) counted over destination nodes)."""
+        w_src = src._state(w_src)
+        w = np.empty(self.n_dofs)
+        ne, no = ctypes.c_int64(), ctypes.c_int64()
+        self._check(self.lib.nsgpu_interpolate(src.ctx, _ptr(w_src), self.ctx, _ptr(w), float(tol), float(padding), ctypes.byref(ne), ctypes.byref(no)),
+                    "interpolate")
+        return w, {"n_extrapolated": ne.value, "n_outside": no.value}
+
+    def interpolate_nonmatching_dev(self, src, w_src_dev, w_dev, tol=1e-12, padding=0.0, counts_dev=None):
+        """``interpolate_nonmatching`` on device vectors, asynchronous on this context's stream (which first waits for src's);
+        counts_dev: None or a device pointer to two int64 (extrapolated, outside)."""
+        ne = no = None
+        if counts_dev is not None:
+            base = counts_dev.value if isinstance(counts_dev, ctypes.c_void_p) else int(counts_dev)
+            ne, no = ctypes.c_void_p(base), ctypes.c_void_p(base + 8)
+        self._check(self.lib.nsgpu_interpolate_dev(src.ctx, w_src_dev, self.ctx, w_dev, float(tol), float(padding), ne, no), "interpolate_dev")
+
     def values_norm(self):
         """Frobenius norm of the resident Jacobian over all ranks' owned rows (a partition-independent checksum)."""
         out = ctypes.c_double()

@@ -33,6 +33,17 @@ struct RowPlan {
   double* d_recv_buf = nullptr;
 };
 
+// Point locator of a context's mesh (locate.cu): per-cell affine maps and a uniform bin grid over the bounding box with, per bin,
+// the ascending list of cells whose box overlaps it.  Depends on the mesh only; built on first use, freed with the mesh.
+struct Locator {
+  double* d_cmap = nullptr;        // per cell gdim + gdim^2 doubles: x0, K (row a = gradient of barycentric coordinate a+1)
+  int64_t* d_bin_ptr = nullptr;    // n_bins + 1
+  int32_t* d_bin_cells = nullptr;
+  double lo[3], inv_h[3];
+  int nb[3];                       // nb[2] = 1 for triangles
+  int64_t n_bins = 0, n_entries = 0;
+};
+
 }  // namespace nsgpu
 
 struct nsgpu_ctx {
@@ -84,7 +95,8 @@ struct nsgpu_ctx {
   void* ilu = nullptr;                         // colouring + factors of the multicolour block ILU(0) preconditioner (ilu.cu)
   void* pilu = nullptr;                        // colouring + factor of the multicolour point ILU(0) preconditioner (pilu.cu)
   void* rowown_plan = nullptr;                 // entity incidence lists + point records of the row-owner kernel (rowown.cu)
-  void* trace = nullptr;                       // locator + velocity tables of the streamline tracer (streamtrace.cu)
+  void* trace = nullptr;                       // velocity tables of the streamline tracer (streamtrace.cu)
+  nsgpu::Locator* locator = nullptr;           // point locator of the mesh (locate.cu)
 
   // internal numbering (renumber.cu): caller local dof d <-> internal dof d_perm[d]; d_perm == nullptr means identity
   int renumber = 1;         // option: 0 never, 1 when the caller's numbering is not vertex-blocked, 2 always
@@ -231,6 +243,9 @@ int rowown_assemble(nsgpu_ctx* ctx, const double* d_xin, bool want_J, bool want_
 void rowown_free(nsgpu_ctx* ctx);
 // streamtrace.cu
 void trace_free(nsgpu_ctx* ctx);
+// locate.cu: the context's locator, built on first use (synchronous); locator_free drops it (nsgpu_set_mesh, nsgpu_destroy)
+int locator_get(nsgpu_ctx* ctx, const Locator** out);
+void locator_free(nsgpu_ctx* ctx);
 // renumber.cu
 int renumber_build(nsgpu_ctx* ctx);
 int renumber_extend_cols(nsgpu_ctx* ctx, int64_t n_extra, const int32_t* leader_local, const int32_t* slot, const int32_t* size,

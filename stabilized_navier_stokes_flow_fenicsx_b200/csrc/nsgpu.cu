@@ -154,6 +154,7 @@ int nsgpu_destroy(nsgpu_ctx* ctx) {
   pilu_free(ctx);
   rowown_free(ctx);
   trace_free(ctx);
+  locator_free(ctx);
   renumber_free(ctx);
   cudaFree(ctx->d_nonfinite);
   if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
@@ -183,6 +184,7 @@ int nsgpu_set_mesh(nsgpu_ctx* ctx, int gdim, int64_t n_nodes, const double* x, i
   ctx->gdim = gdim; ctx->n_nodes = n_nodes; ctx->n_cells_owned = n_cells_owned; ctx->n_cells_total = n_cells_total;
   ctx->pattern_built = false;
   trace_free(ctx);
+  locator_free(ctx);
   for (int k = 0; k < 3; ++k) { ctx->bbox_lo[k] = x[k]; ctx->bbox_hi[k] = x[k]; }
   for (int64_t i = 1; i < n_nodes; ++i)
     for (int k = 0; k < 3; ++k) {

@@ -5,105 +5,20 @@
 // The reference integrates every seed with its own scipy solve_ivp call whose right-hand side queries a dolfinx
 // bounding-box tree and uh.eval through Python (a ThreadPool / round-robin MPI loop over ~40 000 seeds).  Here one
 // thread integrates one seed from start to finish (trace_core.cuh); the per-cell tables it reads are
-//   cmap[cell]  = x0, K        point -> barycentric coordinates (12 doubles)
+//   cmap[cell]  = x0, K        point -> barycentric coordinates (12 doubles)          } the context's Locator (locate.cu),
+//   bins        = uniform grid, per bin the sorted list of cells whose box overlaps it } shared with the point evaluation
 //   cvel[cell]  = c, A         u(x) = c + A x on the cell (12 doubles, rebuilt when the velocity changes)
-//   bins        = uniform grid over the mesh's bounding box; per bin the sorted list of cells whose box overlaps it
-// The bin lists come from a count / scan / fill / radix-sort pass on the device, so the list order (and with it the
-// cell chosen for a point on a shared face) is deterministic.
-#include <cub/cub.cuh>
-
 #include "common.cuh"
 #include "trace_core.cuh"
 
 namespace nsgpu {
 
 struct TracePlan {
-  double* d_cmap = nullptr;
   double* d_cvel = nullptr;
   double* d_u = nullptr;
-  int64_t* d_bin_ptr = nullptr;
-  int32_t* d_bin_cells = nullptr;
-  int64_t n_bins = 0, n_entries = 0;
   bool has_velocity = false;
   TraceField F{};
 };
-
-struct BinGrid {
-  double lo[3], inv_h[3];
-  int nb[3];
-};
-
-__device__ __forceinline__ void cell_bin_range(const BinGrid& G, const double* xg, const int32_t* cv, int* b0, int* b1) {
-  for (int k = 0; k < 3; ++k) {
-    double mn = xg[3 * (int64_t)cv[0] + k], mx = mn;
-    for (int a = 1; a < 4; ++a) {
-      const double v = xg[3 * (int64_t)cv[a] + k];
-      mn = v < mn ? v : mn;
-      mx = v > mx ? v : mx;
-    }
-    // a point within the inside-tolerance of the cell may sit one ulp outside its box: widen by a hair
-    const double pad = 1e-9 / G.inv_h[k];
-    int i0 = (int)floor((mn - pad - G.lo[k]) * G.inv_h[k]), i1 = (int)floor((mx + pad - G.lo[k]) * G.inv_h[k]);
-    i0 = i0 < 0 ? 0 : (i0 >= G.nb[k] ? G.nb[k] - 1 : i0);
-    i1 = i1 < 0 ? 0 : (i1 >= G.nb[k] ? G.nb[k] - 1 : i1);
-    b0[k] = i0; b1[k] = i1;
-  }
-}
-
-__global__ void k_trace_cellmap(int64_t n_cells, BinGrid G, const double* __restrict__ xg, const int32_t* __restrict__ cells,
-                                double* __restrict__ cmap, int64_t* __restrict__ count) {
-  const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (c >= n_cells) return;
-  const int32_t* cv = cells + 4 * c;
-  double x0[3], J[3][3];
-  for (int i = 0; i < 3; ++i) x0[i] = xg[3 * (int64_t)cv[0] + i];
-  for (int i = 0; i < 3; ++i)
-    for (int j = 0; j < 3; ++j) J[i][j] = xg[3 * (int64_t)cv[j + 1] + i] - x0[i];
-  const double c0 = J[1][1] * J[2][2] - J[1][2] * J[2][1];
-  const double c1 = J[1][2] * J[2][0] - J[1][0] * J[2][2];
-  const double c2 = J[1][0] * J[2][1] - J[1][1] * J[2][0];
-  const double id = 1.0 / (J[0][0] * c0 + J[0][1] * c1 + J[0][2] * c2);
-  double* m = cmap + 12 * c;
-  m[0] = x0[0]; m[1] = x0[1]; m[2] = x0[2];
-  m[3] = c0 * id; m[4] = (J[0][2] * J[2][1] - J[0][1] * J[2][2]) * id; m[5] = (J[0][1] * J[1][2] - J[0][2] * J[1][1]) * id;
-  m[6] = c1 * id; m[7] = (J[0][0] * J[2][2] - J[0][2] * J[2][0]) * id; m[8] = (J[0][2] * J[1][0] - J[0][0] * J[1][2]) * id;
-  m[9] = c2 * id; m[10] = (J[0][1] * J[2][0] - J[0][0] * J[2][1]) * id; m[11] = (J[0][0] * J[1][1] - J[0][1] * J[1][0]) * id;
-  int b0[3], b1[3];
-  cell_bin_range(G, xg, cv, b0, b1);
-  count[c] = (int64_t)(b1[0] - b0[0] + 1) * (b1[1] - b0[1] + 1) * (b1[2] - b0[2] + 1);
-}
-
-__global__ void k_trace_fill(int64_t n_cells, BinGrid G, const double* __restrict__ xg, const int32_t* __restrict__ cells,
-                             const int64_t* __restrict__ offset, uint64_t* __restrict__ keys) {
-  const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (c >= n_cells) return;
-  int b0[3], b1[3];
-  cell_bin_range(G, xg, cells + 4 * c, b0, b1);
-  int64_t o = offset[c];
-  for (int k = b0[2]; k <= b1[2]; ++k)
-    for (int j = b0[1]; j <= b1[1]; ++j)
-      for (int i = b0[0]; i <= b1[0]; ++i) {
-        const uint64_t bin = ((uint64_t)k * G.nb[1] + j) * G.nb[0] + i;
-        keys[o++] = (bin << 32) | (uint64_t)(uint32_t)c;
-      }
-}
-
-__global__ void k_trace_binptr(int64_t n_bins, int64_t n_entries, const uint64_t* __restrict__ keys, int64_t* __restrict__ bin_ptr) {
-  const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (b > n_bins) return;
-  const uint64_t want = (uint64_t)b << 32;
-  int64_t lo = 0, hi = n_entries;
-  while (lo < hi) {
-    const int64_t mid = (lo + hi) >> 1;
-    if (keys[mid] < want) lo = mid + 1; else hi = mid;
-  }
-  bin_ptr[b] = lo;
-}
-
-__global__ void k_trace_bincells(int64_t n, const uint64_t* __restrict__ keys, int32_t* __restrict__ out) {
-  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (i < n) out[i] = (int32_t)(keys[i] & 0xffffffffu);
-}
 
 // u(x) = c + A x on each cell from the nodal values:  A = sum_a (u_a - u_0) (x) K_a,  c = u_0 - A x0
 __global__ void k_trace_cellvel(int64_t n_cells, const int32_t* __restrict__ cells, const double* __restrict__ cmap,
@@ -154,85 +69,21 @@ k_trace_run(int64_t n, TraceField F, TraceParams P, const double* __restrict__ s
 void trace_free(nsgpu_ctx* ctx) {
   TracePlan* T = static_cast<TracePlan*>(ctx->trace);
   if (!T) return;
-  cudaFree(T->d_cmap); cudaFree(T->d_cvel); cudaFree(T->d_u); cudaFree(T->d_bin_ptr); cudaFree(T->d_bin_cells);
+  cudaFree(T->d_cvel); cudaFree(T->d_u);
   delete T;
   ctx->trace = nullptr;
 }
 
-static int trace_build(nsgpu_ctx* ctx, double tol) {
-  trace_free(ctx);
+static int trace_build(nsgpu_ctx* ctx) {
+  const Locator* L = nullptr;
+  int rc = locator_get(ctx, &L);
+  if (rc) return rc;
   TracePlan* T = new TracePlan();
   ctx->trace = T;
-  const int64_t nc = ctx->n_cells_total;
-  BinGrid G;
-  double vol = 1.0;
-  for (int k = 0; k < 3; ++k) {
-    const double ext = ctx->bbox_hi[k] - ctx->bbox_lo[k];
-    vol *= ext > 0 ? ext : 1.0;
-  }
-  const double s = 1.5 * cbrt(vol / (double)(nc > 0 ? nc : 1));
-  int64_t n_bins = 1;
-  for (int k = 0; k < 3; ++k) {
-    const double ext = ctx->bbox_hi[k] - ctx->bbox_lo[k];
-    int nb = (int)ceil(ext / s);
-    nb = nb < 1 ? 1 : (nb > 1024 ? 1024 : nb);
-    G.nb[k] = nb;
-    G.lo[k] = ctx->bbox_lo[k];
-    G.inv_h[k] = ext > 0 ? nb / ext : 1.0;
-    n_bins *= nb;
-  }
-  int rc;
-  int64_t* d_count = nullptr;
-  int64_t* d_offset = nullptr;
-  uint64_t* d_keys = nullptr;
-  uint64_t* d_keys2 = nullptr;
-  void* d_tmp = nullptr;
-  auto cleanup = [&]() { cudaFree(d_count); cudaFree(d_offset); cudaFree(d_keys); cudaFree(d_keys2); cudaFree(d_tmp); };
-#define TR_CUDA(call)                                                                                  \
-  do {                                                                                                 \
-    cudaError_t e__ = (call);                                                                          \
-    if (e__ != cudaSuccess) {                                                                          \
-      set_error(ctx, std::string("trace_setup: " #call ": ") + cudaGetErrorString(e__));               \
-      cleanup(); trace_free(ctx);                                                                      \
-      return NSGPU_ECUDA;                                                                              \
-    }                                                                                                  \
-  } while (0)
-  if ((rc = dev_alloc(ctx, &T->d_cmap, 12 * nc)) || (rc = dev_alloc(ctx, &T->d_cvel, 12 * nc)) || (rc = dev_alloc(ctx, &T->d_u, 3 * ctx->n_nodes)) ||
-      (rc = dev_alloc(ctx, &T->d_bin_ptr, n_bins + 1))) { trace_free(ctx); return rc; }
-  TR_CUDA(cudaMalloc(&d_count, sizeof(int64_t) * (nc + 1)));
-  TR_CUDA(cudaMalloc(&d_offset, sizeof(int64_t) * (nc + 1)));
-  TR_CUDA(cudaMemsetAsync(d_count, 0, sizeof(int64_t) * (nc + 1), ctx->stream));
-  const unsigned gc = (unsigned)ceil_div(nc, 128);
-  k_trace_cellmap<<<gc, 128, 0, ctx->stream>>>(nc, G, ctx->d_x, ctx->d_cells, T->d_cmap, d_count);
-  size_t tmp_bytes = 0;
-  TR_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_count, d_offset, nc + 1, ctx->stream));
-  TR_CUDA(cudaMalloc(&d_tmp, tmp_bytes));
-  TR_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, d_count, d_offset, nc + 1, ctx->stream));
-  int64_t n_entries = 0;
-  TR_CUDA(cudaMemcpyAsync(&n_entries, d_offset + nc, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-  TR_CUDA(cudaStreamSynchronize(ctx->stream));
-  TR_CUDA(cudaMalloc(&d_keys, sizeof(uint64_t) * (n_entries > 0 ? n_entries : 1)));
-  TR_CUDA(cudaMalloc(&d_keys2, sizeof(uint64_t) * (n_entries > 0 ? n_entries : 1)));
-  k_trace_fill<<<gc, 128, 0, ctx->stream>>>(nc, G, ctx->d_x, ctx->d_cells, d_offset, d_keys);
-  cudaFree(d_tmp); d_tmp = nullptr;
-  int end_bit = 32;
-  while ((int64_t(1) << (end_bit - 32)) < n_bins) ++end_bit;
-  TR_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, d_keys, d_keys2, n_entries, 0, end_bit, ctx->stream));
-  TR_CUDA(cudaMalloc(&d_tmp, tmp_bytes));
-  TR_CUDA(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, d_keys, d_keys2, n_entries, 0, end_bit, ctx->stream));
-  if ((rc = dev_alloc(ctx, &T->d_bin_cells, n_entries))) { cleanup(); trace_free(ctx); return rc; }
-  k_trace_binptr<<<(unsigned)ceil_div(n_bins + 1, 256), 256, 0, ctx->stream>>>(n_bins, n_entries, d_keys2, T->d_bin_ptr);
-  k_trace_bincells<<<(unsigned)ceil_div(n_entries > 0 ? n_entries : 1, 256), 256, 0, ctx->stream>>>(n_entries, d_keys2, T->d_bin_cells);
-  ctx->launches += 4;
-  TR_CUDA(cudaGetLastError());
-  TR_CUDA(cudaStreamSynchronize(ctx->stream));
-  cleanup();
-#undef TR_CUDA
-  T->n_bins = n_bins; T->n_entries = n_entries;
+  if ((rc = dev_alloc(ctx, &T->d_cvel, 12 * ctx->n_cells_total)) || (rc = dev_alloc(ctx, &T->d_u, 3 * ctx->n_nodes))) { trace_free(ctx); return rc; }
   TraceField& F = T->F;
-  F.cmap = T->d_cmap; F.cvel = T->d_cvel; F.bin_ptr = T->d_bin_ptr; F.bin_cells = T->d_bin_cells;
-  for (int k = 0; k < 3; ++k) { F.lo[k] = G.lo[k]; F.inv_h[k] = G.inv_h[k]; F.nb[k] = G.nb[k]; }
-  F.tol = tol;
+  F.cmap = L->d_cmap; F.cvel = T->d_cvel; F.bin_ptr = L->d_bin_ptr; F.bin_cells = L->d_bin_cells;
+  for (int k = 0; k < 3; ++k) { F.lo[k] = L->lo[k]; F.inv_h[k] = L->inv_h[k]; F.nb[k] = L->nb[k]; }
   return NSGPU_OK;
 }
 
@@ -251,14 +102,15 @@ int nsgpu_trace_setup(nsgpu_ctx* ctx, const double* u_nodes, double tol) {
   NS_REQUIRE(ctx, ctx->gdim == 3 && ctx->n_cells_total > 0, "trace_setup: needs a tetrahedral mesh (nsgpu_set_mesh with gdim 3)");
   NS_REQUIRE(ctx, tol >= 0.0 && tol < 1e-3, "trace_setup: tol must be a small non-negative number");
   TracePlan* T = static_cast<TracePlan*>(ctx->trace);
-  if (!T || T->F.tol != tol) {
-    const int rc = trace_build(ctx, tol);
+  if (!T) {
+    const int rc = trace_build(ctx);
     if (rc) return rc;
     T = static_cast<TracePlan*>(ctx->trace);
   }
+  T->F.tol = tol;
   if (u_nodes) {
     NS_CUDA(ctx, h2d_sync(ctx, T->d_u, u_nodes, sizeof(double) * 3 * ctx->n_nodes));
-    k_trace_cellvel<<<(unsigned)ceil_div(ctx->n_cells_total, 128), 128, 0, ctx->stream>>>(ctx->n_cells_total, ctx->d_cells, T->d_cmap, T->d_u, T->d_cvel);
+    k_trace_cellvel<<<(unsigned)ceil_div(ctx->n_cells_total, 128), 128, 0, ctx->stream>>>(ctx->n_cells_total, ctx->d_cells, T->F.cmap, T->d_u, T->d_cvel);
     ctx->launches += 1;
     NS_CUDA(ctx, cudaGetLastError());
     NS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));

@@ -22,7 +22,8 @@
 
 namespace nsgpu {
 
-// Locator + field tables (device pointers in the library, host pointers in the test harness)
+// Locator + field tables (device pointers in the library, host pointers in the test harness); the locator part is a view of
+// the context's Locator (csrc/locate.cu)
 struct TraceField {
   const double* cmap;      // per cell 12 doubles: x0[3], K[3][3] (row a = gradient of barycentric coordinate a+1)
   const double* cvel;      // per cell 12 doubles: c[3], A[3][3]  with  u(x) = c + A x
@@ -44,33 +45,59 @@ struct TraceParams {
 
 enum { TRACE_FINISHED = 0, TRACE_EVENT_POSITION = 1, TRACE_EVENT_SPEED = 2, TRACE_STEP_TOO_SMALL = -1, TRACE_MAX_STEPS = -2 };
 
-TR_HD bool tr_inside(const TraceField& F, int32_t c, const double* p) {
-  const double* m = F.cmap + 12 * (int64_t)c;
-  const double d0 = p[0] - m[0], d1 = p[1] - m[1], d2 = p[2] - m[2];
-  const double l1 = m[3] * d0 + m[4] * d1 + m[5] * d2;
-  const double l2 = m[6] * d0 + m[7] * d1 + m[8] * d2;
-  const double l3 = m[9] * d0 + m[10] * d1 + m[11] * d2;
-  const double l0 = 1.0 - l1 - l2 - l3;
-  const double t = -F.tol;
-  return l0 >= t && l1 >= t && l2 >= t && l3 >= t;
+// ---- point locator queries (the tables are built by csrc/locate.cu; also used by the point evaluation there) ----
+// cmap row of a cell: x0[GD], then K[GD][GD] with row a = gradient of barycentric coordinate a+1
+template <int GD> TR_HD void loc_bary(const double* cmap, int32_t c, const double* p, double* l) {
+  if constexpr (GD == 3) {
+    const double* m = cmap + 12 * (int64_t)c;
+    const double d0 = p[0] - m[0], d1 = p[1] - m[1], d2 = p[2] - m[2];
+    l[1] = m[3] * d0 + m[4] * d1 + m[5] * d2;
+    l[2] = m[6] * d0 + m[7] * d1 + m[8] * d2;
+    l[3] = m[9] * d0 + m[10] * d1 + m[11] * d2;
+    l[0] = 1.0 - l[1] - l[2] - l[3];
+  } else {
+    const double* m = cmap + 6 * (int64_t)c;
+    const double d0 = p[0] - m[0], d1 = p[1] - m[1];
+    l[1] = m[2] * d0 + m[3] * d1;
+    l[2] = m[4] * d0 + m[5] * d1;
+    l[0] = 1.0 - l[1] - l[2];
+  }
 }
+
+// inside = every barycentric coordinate >= -tol
+template <int GD> TR_HD bool loc_inside(const double* cmap, int32_t c, const double* p, double tol) {
+  double l[GD + 1];
+  loc_bary<GD>(cmap, c, p, l);
+  const double t = -tol;
+  bool in = true;
+  for (int a = 0; a <= GD; ++a) in = in && l[a] >= t;
+  return in;
+}
+
+// lowest-numbered cell of p's bin that holds p; -1 when none does (or p is off the grid).  The grid has one layer in z for GD = 2.
+template <int GD> TR_HD int32_t loc_find(const double* cmap, const int64_t* bin_ptr, const int32_t* bin_cells, const double* lo,
+                                         const double* inv_h, const int* nb, double tol, const double* p) {
+  int b[3] = {0, 0, 0};
+  for (int k = 0; k < GD; ++k) {
+    const double s = (p[k] - lo[k]) * inv_h[k];
+    if (!(s >= 0.0) || s >= (double)nb[k] + 1e-9) return -1;
+    int i = (int)s;
+    b[k] = i >= nb[k] ? nb[k] - 1 : i;
+  }
+  const int64_t bin = ((int64_t)b[2] * nb[1] + b[1]) * nb[0] + b[0];
+  for (int64_t k = bin_ptr[bin]; k < bin_ptr[bin + 1]; ++k) {
+    const int32_t c = bin_cells[k];
+    if (loc_inside<GD>(cmap, c, p, tol)) return c;
+  }
+  return -1;
+}
+
+TR_HD bool tr_inside(const TraceField& F, int32_t c, const double* p) { return loc_inside<3>(F.cmap, c, p, F.tol); }
 
 // cell holding p: the cached cell if it still does, else the lowest-numbered cell of p's bin that does; -1 outside the mesh
 TR_HD int32_t tr_locate(const TraceField& F, const double* p, int32_t hint) {
   if (hint >= 0 && tr_inside(F, hint, p)) return hint;
-  int b[3];
-  for (int k = 0; k < 3; ++k) {
-    const double s = (p[k] - F.lo[k]) * F.inv_h[k];
-    if (!(s >= 0.0) || s >= (double)F.nb[k] + 1e-9) return -1;
-    int i = (int)s;
-    b[k] = i >= F.nb[k] ? F.nb[k] - 1 : i;
-  }
-  const int64_t bin = ((int64_t)b[2] * F.nb[1] + b[1]) * F.nb[0] + b[0];
-  for (int64_t k = F.bin_ptr[bin]; k < F.bin_ptr[bin + 1]; ++k) {
-    const int32_t c = F.bin_cells[k];
-    if (tr_inside(F, c, p)) return c;
-  }
-  return -1;
+  return loc_find<3>(F.cmap, F.bin_ptr, F.bin_cells, F.lo, F.inv_h, F.nb, F.tol, p);
 }
 
 // velfunc / velfunc_reverese: dir * u(p), zero outside the mesh
