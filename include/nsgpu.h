@@ -295,6 +295,33 @@ int nsgpu_interpolate(nsgpu_ctx* src, const double* w_src, nsgpu_ctx* dst, doubl
 int nsgpu_interpolate_dev(nsgpu_ctx* src, const double* w_src_dev, nsgpu_ctx* dst, double* w_dst_dev, double tol, double padding,
                           int64_t* n_extrapolated_dev, int64_t* n_outside_dev);
 
+/* ---- boundary functionals over tagged exterior facets (drag and lift: DFG_2D_Validation.py:193-206, DFG_3D_Validation.py:344-367;
+ *      the inlet / outlet fluxes of the channel and duct drivers' mass-conservation checks) ----------------------------------------
+ * nsgpu_set_facets: the integration domain of ds(subdomain_data=facet_tags), in the format of dolfinx's compute_integration_domains: one
+ *   (cell, local facet, tag) per exterior facet.  Local facet i is the facet opposite vertex i (basix: tets (1,2,3), (0,2,3), (0,1,3),
+ *   (0,1,2); triangles (1,2), (0,2), (0,1)).  Tags in [0, 64); *n_tags_out (may be NULL) = max tag + 1 (with a communicator: the
+ *   largest over the ranks, and the call is collective); output rows are indexed by tag, a tag without facets gives zeros.  Pairs of
+ *   ghost cells (cell >= n_cells_owned) are integrated by the rank that owns the cell, but their dofs still count for the reaction.
+ *   NSGPU_EINVAL, and nothing changes, for NULL arrays, a cell outside [0, n_cells_total), a local facet outside [0, gdim], a tag
+ *   outside [0, 64) or a call before nsgpu_set_mesh / nsgpu_set_space.  A new call replaces the set; nsgpu_set_mesh / nsgpu_set_space
+ *   drop it.
+ * nsgpu_facet_integrals: per tag t, out[t] = [area, int u.n, int p n (gdim), int (grad u) n (gdim), int (grad u)^T n (gdim)]
+ *   (2 + 3 gdim values, (grad u)_ij = du_i/dx_j, n the cell's outward unit normal), with no viscosity applied: the sigma traction
+ *   is nu ((grad u) n + (grad u)^T n) - p n.  Exact for P1 / P2 velocity and P1 pressure (edge-midpoint rule on triangle facets,
+ *   2-point Gauss on segments).
+ * nsgpu_reaction: out[t][c] = sum over the velocity dofs of component c in the closure of the facets of tag t (vertices, plus edges
+ *   for P2; a dof on facets of two tags counts for both, as locate_dofs_topological(ft.find(tag)) per tag) of the UNCONSTRAINED
+ *   residual of the current form (no lifting, no set_bc) assembled over the owned cells: the consistent reaction, the accurate drag /
+ *   lift for P1.  The force the fluid exerts on the tagged boundary is -out[t].
+ * w_local: n_owned + n_ghost values in the caller's numbering.  Rows are reduced in a fixed order (bitwise reproducible) and summed
+ * over the ranks when a communicator is attached (collective).  The _dev variants take device pointers and are asynchronous on the
+ * context's stream. */
+int nsgpu_set_facets(nsgpu_ctx* ctx, int64_t n, const int32_t* cell, const int32_t* local_facet, const int32_t* tag, int32_t* n_tags_out);
+int nsgpu_facet_integrals(nsgpu_ctx* ctx, const double* w_local, double* out /* n_tags x (2 + 3 gdim) */);
+int nsgpu_facet_integrals_dev(nsgpu_ctx* ctx, const double* w_local_dev, double* out_dev);
+int nsgpu_reaction(nsgpu_ctx* ctx, const double* w_local, double* out /* n_tags x gdim */);
+int nsgpu_reaction_dev(nsgpu_ctx* ctx, const double* w_local_dev, double* out_dev);
+
 #ifdef __cplusplus
 }
 #endif

@@ -88,6 +88,11 @@ SIGNATURES = {
     "nsgpu_eval_dev": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
     "nsgpu_interpolate": (ctypes.c_int, [c_ctx, ctypes.c_void_p, c_ctx, ctypes.c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
     "nsgpu_interpolate_dev": (ctypes.c_int, [c_ctx, ctypes.c_void_p, c_ctx, ctypes.c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
+    "nsgpu_set_facets": (ctypes.c_int, [c_ctx, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, c_i32p]),
+    "nsgpu_facet_integrals": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.c_void_p]),
+    "nsgpu_facet_integrals_dev": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.c_void_p]),
+    "nsgpu_reaction": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.c_void_p]),
+    "nsgpu_reaction_dev": (ctypes.c_int, [c_ctx, ctypes.c_void_p, ctypes.c_void_p]),
 }
 
 

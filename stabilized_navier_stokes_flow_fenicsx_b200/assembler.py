@@ -50,6 +50,7 @@ class NSAssembler:
         self.n_cols = self.n_dofs
         self.nnz = None
         self.n_rows = None
+        self.n_tags = 0
 
     # ------------------------------------------------------------------ plumbing
     def _check(self, rc, what):
@@ -373,6 +374,47 @@ class NSAssembler:
             base = counts_dev.value if isinstance(counts_dev, ctypes.c_void_p) else int(counts_dev)
             ne, no = ctypes.c_void_p(base), ctypes.c_void_p(base + 8)
         self._check(self.lib.nsgpu_interpolate_dev(src.ctx, w_src_dev, self.ctx, w_dev, float(tol), float(padding), ne, no), "interpolate_dev")
+
+    # ------------------------------------------------------------------ boundary functionals over tagged facets
+    def set_facets(self, cells, local_facets, tags):
+        """Integration domain of ``ds(subdomain_data=facet_tags)``: one (cell, local facet, tag) per exterior facet (dolfinx's
+        compute_integration_domains; local facet i is opposite vertex i; ``gmsh_io.facet_integration_domain`` builds them from
+        tagged facets).  Tags in [0, 64).  Facets of ghost cells are integrated by the owning rank.  Returns n_tags = max tag + 1."""
+        c = np.ascontiguousarray(cells, dtype=np.int32).ravel()
+        lf = np.ascontiguousarray(local_facets, dtype=np.int32).ravel()
+        t = np.ascontiguousarray(tags, dtype=np.int32).ravel()
+        if not (len(c) == len(lf) == len(t)):
+            raise ValueError("cells, local_facets and tags must have the same length")
+        n = ctypes.c_int32()
+        self._check(self.lib.nsgpu_set_facets(self.ctx, len(c), _ptr(c), _ptr(lf), _ptr(t), ctypes.byref(n)), "set_facets")
+        self.n_tags = n.value
+        return self.n_tags
+
+    def facet_integrals(self, w):
+        """Per tag: [area, int u.n, int p n (gdim), int (grad u) n (gdim), int (grad u)^T n (gdim)] with n the outward unit normal,
+        (grad u)_ij = du_i/dx_j, no viscosity applied; returns (n_tags, 2 + 3 gdim).  The force of the fluid on the tagged
+        boundary by the Cauchy stress is -(nu (row[2+g:2+2g] + row[2+2g:]) - row[2:2+g])."""
+        w = self._state(w)
+        out = np.empty((self.n_tags, 2 + 3 * self.gdim))
+        self._check(self.lib.nsgpu_facet_integrals(self.ctx, _ptr(w), _ptr(out)), "facet_integrals")
+        return out
+
+    def facet_integrals_dev(self, w_dev, out_dev):
+        """``facet_integrals`` on device arrays (out: n_tags x (2 + 3 gdim) doubles); asynchronous on the context's stream."""
+        self._check(self.lib.nsgpu_facet_integrals_dev(self.ctx, w_dev, out_dev), "facet_integrals_dev")
+
+    def reaction(self, w):
+        """Per tag and velocity component: the unconstrained residual of the current form (no lifting, no set_bc) summed over the
+        velocity dofs of the tagged facets (vertices, plus edges for P2); returns (n_tags, gdim).  The force of the fluid on the
+        tagged boundary is -reaction (the consistent drag / lift)."""
+        w = self._state(w)
+        out = np.empty((self.n_tags, self.gdim))
+        self._check(self.lib.nsgpu_reaction(self.ctx, _ptr(w), _ptr(out)), "reaction")
+        return out
+
+    def reaction_dev(self, w_dev, out_dev):
+        """``reaction`` on device arrays (out: n_tags x gdim doubles); asynchronous on the context's stream."""
+        self._check(self.lib.nsgpu_reaction_dev(self.ctx, w_dev, out_dev), "reaction_dev")
 
     def values_norm(self):
         """Frobenius norm of the resident Jacobian over all ranks' owned rows (a partition-independent checksum)."""

@@ -97,6 +97,7 @@ struct nsgpu_ctx {
   void* rowown_plan = nullptr;                 // entity incidence lists + point records of the row-owner kernel (rowown.cu)
   void* trace = nullptr;                       // velocity tables of the streamline tracer (streamtrace.cu)
   nsgpu::Locator* locator = nullptr;           // point locator of the mesh (locate.cu)
+  void* boundary = nullptr;                    // tagged facets of the boundary functionals (boundary.cu)
 
   // internal numbering (renumber.cu): caller local dof d <-> internal dof d_perm[d]; d_perm == nullptr means identity
   int renumber = 1;         // option: 0 never, 1 when the caller's numbering is not vertex-blocked, 2 always
@@ -246,6 +247,8 @@ void trace_free(nsgpu_ctx* ctx);
 // locate.cu: the context's locator, built on first use (synchronous); locator_free drops it (nsgpu_set_mesh, nsgpu_destroy)
 int locator_get(nsgpu_ctx* ctx, const Locator** out);
 void locator_free(nsgpu_ctx* ctx);
+// boundary.cu: drops the tagged facets of nsgpu_set_facets (nsgpu_set_mesh, nsgpu_set_space, nsgpu_destroy)
+void boundary_free(nsgpu_ctx* ctx);
 // renumber.cu
 int renumber_build(nsgpu_ctx* ctx);
 int renumber_extend_cols(nsgpu_ctx* ctx, int64_t n_extra, const int32_t* leader_local, const int32_t* slot, const int32_t* size,

@@ -155,6 +155,7 @@ int nsgpu_destroy(nsgpu_ctx* ctx) {
   rowown_free(ctx);
   trace_free(ctx);
   locator_free(ctx);
+  boundary_free(ctx);
   renumber_free(ctx);
   cudaFree(ctx->d_nonfinite);
   if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
@@ -185,6 +186,7 @@ int nsgpu_set_mesh(nsgpu_ctx* ctx, int gdim, int64_t n_nodes, const double* x, i
   ctx->pattern_built = false;
   trace_free(ctx);
   locator_free(ctx);
+  boundary_free(ctx);
   for (int k = 0; k < 3; ++k) { ctx->bbox_lo[k] = x[k]; ctx->bbox_hi[k] = x[k]; }
   for (int64_t i = 1; i < n_nodes; ++i)
     for (int k = 0; k < 3; ++k) {
@@ -216,6 +218,7 @@ int nsgpu_set_space(nsgpu_ctx* ctx, int vdeg, const int32_t* dofmap, int64_t n_d
   ctx->extra_rows.clear(); ctx->extra_cols.clear();
   ctx->pattern_built = false;
   ctx->has_bc = false;
+  boundary_free(ctx);
   int rc;
   if ((rc = dev_alloc(ctx, &ctx->d_dofmap, ctx->n_cells_total * ctx->nd))) return rc;
   NS_CUDA(ctx, h2d_sync(ctx, ctx->d_dofmap, dofmap, sizeof(int32_t) * ctx->n_cells_total * ctx->nd));

@@ -146,6 +146,37 @@ def boundary_facets(mesh):
     return uniq[cnt == 1].astype(np.int32)
 
 
+def facet_integration_domain(mesh, facets, facet_tags):
+    """The (cell, local facet, tag) triples of ``ds(subdomain_data=facet_tags)`` for the tagged facets of ``read_msh`` /
+    ``boundary_facets`` (what dolfinx's compute_integration_domains gives; local facet i is the facet opposite vertex i).
+    Raises ValueError for a facet that belongs to no cell or to two cells (an interior facet)."""
+    gd = mesh.gdim
+    loc = ((1, 2, 3), (0, 2, 3), (0, 1, 3), (0, 1, 2)) if gd == 3 else ((1, 2), (0, 2), (0, 1))
+    nc = mesh.n_cells
+    allf = np.sort(np.concatenate([mesh.cells[:, f] for f in loc]).astype(np.int64), axis=1)
+    owner = np.arange(len(loc) * nc, dtype=np.int64)                        # row k: cell k % nc, local facet k // nc
+    order = np.lexsort(allf.T[::-1])
+    allf, owner = allf[order], owner[order]
+    want = np.sort(np.asarray(facets, dtype=np.int64).reshape(-1, gd), axis=1)
+    tags = np.asarray(facet_tags, dtype=np.int32).ravel()
+    if len(tags) != len(want):
+        raise ValueError("facets and facet_tags differ in length")
+    nv = max(int(mesh.n_vertices), 1)
+    both = np.concatenate([allf, want])
+    k = both[:, 0] * nv + both[:, 1]                                       # vertex pairs, then triples through the pair's rank
+    if gd == 3:
+        k = np.unique(k, return_inverse=True)[1].ravel().astype(np.int64) * nv + both[:, 2]
+    ka, kw = k[: len(allf)], k[len(allf):]
+    lo, hi = np.searchsorted(ka, kw, "left"), np.searchsorted(ka, kw, "right")
+    cnt = hi - lo
+    if (cnt == 0).any():
+        raise ValueError(f"facet {want[np.flatnonzero(cnt == 0)[0]].tolist()} belongs to no cell")
+    if (cnt > 1).any():
+        raise ValueError(f"facet {want[np.flatnonzero(cnt > 1)[0]].tolist()} is shared by two cells (interior facet)")
+    k = owner[lo]
+    return (k % nc).astype(np.int32), (k // nc).astype(np.int32), tags.copy()
+
+
 def facet_dofs(space, facets, facet_tags, marker, sub="velocity"):
     """locate_dofs_topological((W.sub(i), V), tdim - 1, ft.find(marker)) for the mixed space of mesh.mixed_space:
     velocity -> all components on the vertices (and, for P2, the edges) of the marked facets; pressure -> the vertices."""
