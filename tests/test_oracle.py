@@ -36,7 +36,10 @@ FORMS = [
     ("ugn_p2_tri", dict(flavour=1, gdim=2, vdeg=2, nu=0.01)),
     ("ugn_p1_tet", dict(flavour=1, gdim=3, vdeg=1, nu=0.01)),
     ("gmetric_p1_tri", dict(flavour=0, gdim=2, vdeg=1, nu=0.05)),
-]
+    ("gmetric_p2_tri", dict(flavour=0, gdim=2, vdeg=2, nu=0.05)),
+    ("ugn_p2_tet", dict(flavour=1, gdim=3, vdeg=2, nu=0.01)),
+] + [(f"stokes_{v}_p{k}_{c}", dict(flavour=2, gdim=g, vdeg=k, nu=1.0, alpha=a, sp=s, beta=b))
+     for v, a, s, b in (("pspg", 1.0, 1.0, 0.2), ("plain", 0.7, -1.0, 0.0)) for k in (1, 2) for c, g in (("tri", 2), ("tet", 3))]
 
 
 def _rand_cell(rng, gd, scale=0.1):
