@@ -273,9 +273,27 @@ int nsgpu_trace_run(nsgpu_ctx* ctx, int64_t n, const double* seeds, int reverse,
  *      overlaps, the one at the smallest Euclidean distance from p to the closed cell (ties to the lower cell number), accepted when
  *      that distance is <= padding; that cell's polynomials are evaluated at p;
  *   3. otherwise outside: the values are 0.
- * Single rank only: both contexts must have one rank (NSGPU_EUNSUPPORTED otherwise; distributed point ownership, dolfinx's
- * determine_point_ownership, is not implemented).  NSGPU_EINVAL for NULL arrays, a negative tol or padding, a context without
- * mesh and space, differing gdim or contexts on different devices; nothing is changed then.
+ * NSGPU_EINVAL for NULL arrays, a negative tol or padding, a context without mesh and space, differing gdim or contexts on different
+ * devices; nothing is changed then.
+ *
+ * Several ranks (a context with a communicator, nsgpu_comm_init; dolfinx's determine_point_ownership): the four calls are collective.
+ * Every rank calls them with its own points (n may differ between ranks, or be 0) and the same tol and padding.  Only owned cells
+ * (c < n_cells_owned) hold points.  A point of the calling rank is resolved by:
+ *   1. local first: inside an owned cell of the calling rank, by rule 1 above; such points are never sent to another rank;
+ *   2. otherwise inside elsewhere: the lowest rank with an owned cell that holds the point, and that rank's lowest such cell;
+ *   3. only when padding > 0 and 1-2 fail: over every rank's owned cells the smallest exact point-to-cell distance, ties to the lower
+ *      rank, then to the lower cell, accepted when <= padding; that cell's polynomials are evaluated at the point;
+ *   4. otherwise the values are 0.
+ * The cell codes keep their meaning (c, -2 - c, -1); c is in the numbering of the rank that resolved the point.  Because of "local
+ * first" a point on a partition interface can take its value from different cells depending on which rank asks; for a continuous
+ * field the difference is rounding only.
+ * nsgpu_interpolate on several ranks: the destination rank's owned nodes (first velocity dof, caller numbering, < n_owned) are the
+ * points, evaluated over the source's communicator; the values go to every owned dof at the node, then the ghost entries are
+ * refreshed through the destination's halo plan (nsgpu_set_halo; NSGPU_EINVAL for a destination with ghost dofs and no plan).
+ * n_extrapolated / n_outside are summed over the ranks.  src and dst must have the same nranks and rank and the same device.
+ * Argument checks are local; then one allreduce agrees on a status before any exchange, so every rank returns the same code (the
+ * first failing rank's; NSGPU_EINVAL when tol or padding differ between ranks) and the contexts stay usable.  On several ranks the
+ * _dev variants synchronise their stream: the message sizes have to reach the host.
  *
  * nsgpu_eval: w_local (n_owned + n_ghost values, caller numbering) at n points (n x 3; z ignored on triangles).  values: n x (gdim+1),
  *   the velocity components then the pressure.  cell (may be NULL): c when the point is inside cell c, -2 - c when extrapolated
@@ -284,8 +302,8 @@ int nsgpu_trace_run(nsgpu_ctx* ctx, int64_t n, const double* seeds, int reverse,
  *   source function w_src evaluated at the dof's node (vertices; edge midpoints 0.5 (xa + xb) for P2), each node located once.
  *   The meshes may differ in resolution, cell order, numbering and velocity degree (P1-P1 -> P2-P1 is allowed); gdim must agree.
  *   n_extrapolated / n_outside (may be NULL): destination nodes that took step 2 / step 3.
- * The _dev variants take device pointers (the counts too) and are asynchronous on the stream of ctx / dst; dst's stream first waits
- * for the work queued on src's.  The first call on a mesh builds its locator (synchronous). */
+ * The _dev variants take device pointers (the counts too) and are asynchronous on the stream of ctx / dst (on one rank); dst's stream
+ * first waits for the work queued on src's.  The first call on a mesh builds its locator (synchronous). */
 int nsgpu_eval(nsgpu_ctx* ctx, const double* w_local, int64_t n, const double* points, double tol, double padding, double* values,
                int32_t* cell);
 int nsgpu_eval_dev(nsgpu_ctx* ctx, const double* w_local_dev, int64_t n, const double* points_dev, double tol, double padding,

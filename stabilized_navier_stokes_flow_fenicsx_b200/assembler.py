@@ -340,7 +340,12 @@ class NSAssembler:
     def eval(self, w, points, tol=1e-12, padding=0.0):
         """Function.eval of the mixed function w (caller numbering) at points (n, 3): returns (values (n, gdim + 1) = velocity
         components then pressure, cells (n,) int32).  cells: c inside cell c (lowest-numbered cell with every barycentric coordinate
-        >= -tol), -2 - c extrapolated from the nearest cell c within ``padding``, -1 outside (values 0).  One rank only."""
+        >= -tol), -2 - c extrapolated from the nearest cell c within ``padding``, -1 outside (values 0).
+
+        On a context with a communicator the call is collective: every rank passes its own points (any number, also none) and the
+        same tol and padding; only owned cells hold points.  A point inside an owned cell of the calling rank stays there; otherwise
+        the lowest rank with an owned cell holding it answers; otherwise (padding > 0) the nearest owned cell over all ranks within
+        ``padding`` (ties to the lower rank).  Cell numbers are those of the answering rank."""
         w = self._state(w)
         p = np.ascontiguousarray(points, dtype=np.float64)
         if p.ndim != 2 or p.shape[1] != 3:
@@ -352,13 +357,17 @@ class NSAssembler:
 
     def eval_dev(self, w_dev, n, points_dev, values_dev, cells_dev=None, tol=1e-12, padding=0.0):
         """``eval`` on device arrays (w: n_owned + n_ghost, points: n x 3, values: n x (gdim + 1) doubles, cells: n int32 or None);
-        asynchronous on the context's stream."""
+        asynchronous on the context's stream on one rank; collective and synchronous on several (see ``eval``)."""
         self._check(self.lib.nsgpu_eval_dev(self.ctx, w_dev, int(n), points_dev, float(tol), float(padding), values_dev, cells_dev), "eval_dev")
 
     def interpolate_nonmatching(self, src, w_src, tol=1e-12, padding=0.0):
         """Function.interpolate_nonmatching onto this (destination) space: every dof gets the source function ``w_src`` of the
         NSAssembler ``src`` (another mesh of the same gdim, any velocity degree) evaluated at the dof's node, with the location rule
-        of ``eval``.  Returns (w (n_owned + n_ghost), info = dict(n_extrapolated, n_outside) counted over destination nodes)."""
+        of ``eval``.  Returns (w (n_owned + n_ghost), info = dict(n_extrapolated, n_outside) counted over destination nodes).
+
+        On several ranks (both contexts with communicators of the same size, the destination with its halo plan) the call is
+        collective: each rank's owned destination nodes are evaluated over the source's ranks, the ghost entries are refreshed from
+        their owners, and the counts are summed over the ranks."""
         w_src = src._state(w_src)
         w = np.empty(self.n_dofs)
         ne, no = ctypes.c_int64(), ctypes.c_int64()
@@ -368,7 +377,7 @@ class NSAssembler:
 
     def interpolate_nonmatching_dev(self, src, w_src_dev, w_dev, tol=1e-12, padding=0.0, counts_dev=None):
         """``interpolate_nonmatching`` on device vectors, asynchronous on this context's stream (which first waits for src's);
-        counts_dev: None or a device pointer to two int64 (extrapolated, outside)."""
+        counts_dev: None or a device pointer to two int64 (extrapolated, outside).  Synchronous on several ranks."""
         ne = no = None
         if counts_dev is not None:
             base = counts_dev.value if isinstance(counts_dev, ctypes.c_void_p) else int(counts_dev)

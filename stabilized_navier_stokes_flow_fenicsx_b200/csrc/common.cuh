@@ -212,6 +212,10 @@ int rows_exchange_begin(nsgpu_ctx* ctx, cudaStream_t stream);
 int rows_exchange_end(nsgpu_ctx* ctx);
 void halo_free(nsgpu_ctx* ctx);
 int allreduce_sum(nsgpu_ctx* ctx, double* d_buf, int n);
+// grouped ncclSend / ncclRecv of double segments: sbuf[sptr[k], sptr[k+1]) to ranks[k], rbuf[rptr[k], rptr[k+1]) from ranks[k];
+// empty segments are skipped; stream nullptr = the context's
+int exchange(nsgpu_ctx* ctx, const std::vector<int>& ranks, const std::vector<int64_t>& sptr, const double* sbuf,
+             const std::vector<int64_t>& rptr, double* rbuf, cudaStream_t stream = nullptr);
 // krylov.cu
 int tfqmr_impl(nsgpu_ctx* ctx, const double* d_b, double* d_x, double rtol, double atol, int max_it, int pc, bool zero_guess, int* its_out,
                double* rnorm_out, double* r0norm_out);

@@ -84,8 +84,8 @@ __global__ void k_scatter_add64(int64_t n, const int64_t* __restrict__ pos, cons
 static inline unsigned g256(int64_t n) { return (unsigned)ceil_div(n > 0 ? n : 1, 256); }
 
 // exchange: send sbuf segments (sptr) to neighbours, receive rbuf segments (rptr)
-static int exchange(nsgpu_ctx* ctx, const std::vector<int>& ranks, const std::vector<int64_t>& sptr, const double* sbuf,
-                    const std::vector<int64_t>& rptr, double* rbuf, cudaStream_t stream = nullptr) {
+int exchange(nsgpu_ctx* ctx, const std::vector<int>& ranks, const std::vector<int64_t>& sptr, const double* sbuf,
+             const std::vector<int64_t>& rptr, double* rbuf, cudaStream_t stream) {
   if (!stream) stream = ctx->stream;
   std::string why;
   NcclApi* api = nccl_api(&why);

@@ -74,9 +74,10 @@ template <int GD> TR_HD bool loc_inside(const double* cmap, int32_t c, const dou
   return in;
 }
 
-// lowest-numbered cell of p's bin that holds p; -1 when none does (or p is off the grid).  The grid has one layer in z for GD = 2.
+// lowest-numbered cell below n_bound of p's bin that holds p; -1 when none does (or p is off the grid).  The grid has one layer in z
+// for GD = 2.  The bin lists are ascending, so the scan stops at the first cell >= n_bound (several ranks: the owned cells only).
 template <int GD> TR_HD int32_t loc_find(const double* cmap, const int64_t* bin_ptr, const int32_t* bin_cells, const double* lo,
-                                         const double* inv_h, const int* nb, double tol, const double* p) {
+                                         const double* inv_h, const int* nb, int32_t n_bound, double tol, const double* p) {
   int b[3] = {0, 0, 0};
   for (int k = 0; k < GD; ++k) {
     const double s = (p[k] - lo[k]) * inv_h[k];
@@ -87,6 +88,7 @@ template <int GD> TR_HD int32_t loc_find(const double* cmap, const int64_t* bin_
   const int64_t bin = ((int64_t)b[2] * nb[1] + b[1]) * nb[0] + b[0];
   for (int64_t k = bin_ptr[bin]; k < bin_ptr[bin + 1]; ++k) {
     const int32_t c = bin_cells[k];
+    if (c >= n_bound) break;
     if (loc_inside<GD>(cmap, c, p, tol)) return c;
   }
   return -1;
@@ -97,7 +99,7 @@ TR_HD bool tr_inside(const TraceField& F, int32_t c, const double* p) { return l
 // cell holding p: the cached cell if it still does, else the lowest-numbered cell of p's bin that does; -1 outside the mesh
 TR_HD int32_t tr_locate(const TraceField& F, const double* p, int32_t hint) {
   if (hint >= 0 && tr_inside(F, hint, p)) return hint;
-  return loc_find<3>(F.cmap, F.bin_ptr, F.bin_cells, F.lo, F.inv_h, F.nb, F.tol, p);
+  return loc_find<3>(F.cmap, F.bin_ptr, F.bin_cells, F.lo, F.inv_h, F.nb, INT32_MAX, F.tol, p);   // every cell of the mesh
 }
 
 // velfunc / velfunc_reverese: dir * u(p), zero outside the mesh

@@ -224,6 +224,51 @@ def duct_partition(n_cross, n_long, rank, size, length=4.0, seed=1234, noise=1e-
                      l2g, w, bcs, {"k0": k0, "k1": k1, "plane": plane})
 
 
+def partition_cells(mesh, space, cell_rank, rank, size, w=None, bcs=None):
+    """Partition of any mesh and mixed space (tets or triangles, P1-P1 or P2-P1) by a given cell -> rank map, in the layout of
+    ``duct_partition``: the owned cells are those with ``cell_rank == rank`` (no ghost cells), each dof is owned by the lowest rank
+    among the cells that contain it, global dofs are numbered contiguously by rank (ascending serial dof within a rank), and
+    locally the owned dofs come first, then the ghosts, each in global order.  ``w`` (serial numbering) and ``bcs`` (list of
+    (dofs, values) in serial numbering) are mapped to the local numbering; ``meta["serial_dof"]`` is the serial dof of every local
+    dof."""
+    cell_rank = np.asarray(cell_rank, dtype=np.int64)
+    if cell_rank.shape != (mesh.n_cells,) or cell_rank.min() < 0 or cell_rank.max() >= size:
+        raise ValueError("cell_rank must give a rank in [0, size) for every cell")
+    dm = np.asarray(space.dofmap, dtype=np.int64)
+    owner = np.full(space.n_dofs, size, dtype=np.int64)
+    np.minimum.at(owner, dm, np.broadcast_to(cell_rank[:, None], dm.shape))
+    serial_of_global = np.argsort(owner, kind="stable")                 # global dof -> serial dof
+    global_of_serial = np.empty(space.n_dofs, dtype=np.int64)
+    global_of_serial[serial_of_global] = np.arange(space.n_dofs)
+    global_offset = int((owner < rank).sum())
+    own_cells = np.nonzero(cell_rank == rank)[0]
+    if own_cells.size == 0:
+        raise ValueError(f"rank {rank} owns no cell")
+    local_serial = np.unique(dm[own_cells])
+    mine = owner[local_serial] == rank
+    owned, ghost = local_serial[mine], local_serial[~mine]
+    owned = owned[np.argsort(global_of_serial[owned])]
+    ghost = ghost[np.argsort(global_of_serial[ghost])]
+    serial_dof = np.concatenate([owned, ghost])
+    local_of_serial = np.full(space.n_dofs, -1, dtype=np.int64)
+    local_of_serial[serial_dof] = np.arange(len(serial_dof))
+    verts = np.unique(mesh.cells[own_cells])
+    local_vertex = np.full(mesh.n_vertices, -1, dtype=np.int64)
+    local_vertex[verts] = np.arange(len(verts))
+    cells = local_vertex[mesh.cells[own_cells]].astype(np.int32)
+    dofmap = local_of_serial[dm[own_cells]].astype(np.int32)
+    l2g = global_of_serial[serial_dof]
+    n_owned, n_ghost = len(owned), len(ghost)
+    w_local = None if w is None else np.asarray(w, dtype=np.float64)[serial_dof]
+    bcs_local = []
+    for dofs, vals in (bcs or []):
+        ld = local_of_serial[np.asarray(dofs, dtype=np.int64)]
+        keep = ld >= 0
+        bcs_local.append((ld[keep].astype(np.int32), np.asarray(vals, dtype=np.float64)[keep]))
+    return Partition(rank, size, mesh.x[verts], cells, dofmap, len(own_cells), n_owned, n_ghost, global_offset, l2g[n_owned:],
+                     owner[ghost].astype(np.int32), l2g, w_local, bcs_local, {"serial_dof": serial_dof, "cells": own_cells})
+
+
 # ------------------------------------------------------------------------------------------------ plans
 def entity_tables(dofmap, gdim, vdeg, n_dofs):
     """leader / slot / size of every local dof: dofs on one mesh entity (vertex: gdim velocity components +
