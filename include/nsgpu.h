@@ -122,7 +122,9 @@ int nsgpu_spmv(nsgpu_ctx* ctx, const double* x_local, double* y_owned);
  *   pc: 0 none, 1 Jacobi, 4 = 4x4 block Jacobi over the dofs of one P1-P1 vertex (falls back to 1 elsewhere),
  *       5 = multicolour 4x4-block ILU(0), block Jacobi over the ranks (P1-P1 tets; NSGPU_EUNSUPPORTED elsewhere),
  *       6 = multicolour point ILU(0), block Jacobi over the ranks, any space (velocity dofs eliminated before pressure dofs;
- *           NSGPU_EZEROPIVOT on a zero pivot).
+ *           NSGPU_EZEROPIVOT on a zero pivot),
+ *       7 = point ILU(0) in the caller's order of the owned dofs (PETSc's natural order), block Jacobi over the ranks, any space
+ *           (NSGPU_EZEROPIVOT on a zero pivot).
  *   zero_guess != 0 ignores the incoming x (PETSc's default initial guess).
  * Stops when the quasi-residual bound tau*sqrt(m+1) <= max(rtol * ||b||, atol) (PETSc's default test) or after max_it iterations;
  * *its_out = iterations done, *rnorm_out = TRUE residual norm ||b - A x|| at exit, *r0norm_out = ||b - A x0||.
@@ -150,6 +152,14 @@ int nsgpu_ilu_colours(nsgpu_ctx* ctx, int32_t* colour /* n_owned / 4, may be NUL
  * (within a colour the order does not change the factor); for tests. */
 int nsgpu_pilu_apply(nsgpu_ctx* ctx, int refactor, const double* r_owned, double* z_owned);
 int nsgpu_pilu_colours(nsgpu_ctx* ctx, int32_t* colour /* n_owned, may be NULL */, int32_t* n_colours, int32_t* n_velocity_colours);
+/* Point ILU(0) of the resident Jacobian eliminated in the caller's order of the owned dofs (pc = 7 of nsgpu_tfqmr*): the factor PETSc's
+ * default PC computes on the AIJ matrix in its natural order, block Jacobi over the ranks.  No colouring: one launch factorises, one
+ * launch per sweep applies, rows waiting on the rows they depend on.  nsgpu_nilu_apply = PCApply on host vectors in the caller's
+ * numbering, as nsgpu_pilu_apply; NSGPU_EZEROPIVOT names the smallest row (caller's numbering) with a zero or non-finite pivot, agreed
+ * over the ranks.  nsgpu_nilu_depth: the number of levels (rows on the longest dependency path) of the forward and the backward
+ * sweep, which sets their time. */
+int nsgpu_nilu_apply(nsgpu_ctx* ctx, int refactor, const double* r_owned, double* z_owned);
+int nsgpu_nilu_depth(nsgpu_ctx* ctx, int32_t* depth_lower, int32_t* depth_upper);
 int nsgpu_axpy_dev(nsgpu_ctx* ctx, double a, const double* x_dev, double* y_dev);
 int nsgpu_norm_dev(nsgpu_ctx* ctx, const double* x_dev, double* out);
 /* VecDot over the owned entries, reduced over all ranks (the initial slope F . J dx of SNES' backtracking line search). */

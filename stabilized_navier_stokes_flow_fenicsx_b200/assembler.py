@@ -205,7 +205,8 @@ class NSAssembler:
     def tfqmr(self, b, x0=None, rtol=1e-8, atol=0.0, max_it=1000, pc=4):
         """KSPSolve with KSPTFQMR on the resident Jacobian (NavierStokesChannelFlow.py:77, :282-285), fully on the device.
         pc: 0 none, 1 Jacobi, 4 4x4 vertex-block Jacobi (P1-P1 tets, else 1), 5 multicolour block ILU(0) (P1-P1 tets only),
-        6 multicolour point ILU(0) (any space; NsgpuError "zero pivot" when a pivot vanishes).
+        6 multicolour point ILU(0) (any space; NsgpuError "zero pivot" when a pivot vanishes), 7 point ILU(0) in the caller's
+        order of the dofs, PETSc's natural order (any space; NsgpuError "zero pivot" naming the first such row).
         Returns (x_owned, info) with info = dict(its, rnorm = true ||b - A x||, r0norm)."""
         b = np.ascontiguousarray(b, dtype=np.float64)
         x = np.zeros(self.n_owned) if x0 is None else np.array(x0[: self.n_owned], dtype=np.float64)
@@ -254,6 +255,22 @@ class NSAssembler:
         self._check(self.lib.nsgpu_pilu_colours(self.ctx, _ptr(col), ctypes.byref(n), ctypes.byref(nv)), "pilu_colours")
         return col, n.value, nv.value
 
+    def nilu_apply(self, r, refactor=True):
+        """PCApply of the point ILU(0) in the caller's order (pc = 7) on a host vector in the caller's numbering: z = U^-1 L^-1 r."""
+        r = np.ascontiguousarray(r, dtype=np.float64)
+        if r.size < self.n_owned:
+            raise ValueError(f"nilu_apply needs the {self.n_owned} owned entries")
+        z = np.empty(self.n_owned)
+        self._check(self.lib.nsgpu_nilu_apply(self.ctx, 1 if refactor else 0, _ptr(r), _ptr(z)), "nilu_apply")
+        return z
+
+    def nilu_depth(self):
+        """(levels of the forward sweep, levels of the backward sweep) of the caller's-order ILU(0): rows on the longest path of
+        each dependency DAG."""
+        lo, up = ctypes.c_int32(), ctypes.c_int32()
+        self._check(self.lib.nsgpu_nilu_depth(self.ctx, ctypes.byref(lo), ctypes.byref(up)), "nilu_depth")
+        return lo.value, up.value
+
     def axpy_dev(self, a, x_dev, y_dev):
         self._check(self.lib.nsgpu_axpy_dev(self.ctx, float(a), x_dev, y_dev), "axpy_dev")
 
@@ -272,8 +289,8 @@ class NSAssembler:
         NavierStokesChannelFlow.py:286-291): F and J from the assembly kernels, dw from TFQMR, w -= lambda dw.
         ``linesearch``: "bt" = PETSc's default for newtonls (SNESLineSearchBT: sufficient decrease alpha = 1e-4 on
         1/2 ||F||^2, quadratic then cubic backtracking, steps clipped to [0.1, 0.5] of the previous one, at most 40), or
-        "basic" (full steps).  ``pc``: the preconditioner of the TFQMR solves, as in ``tfqmr`` (6, the point ILU(0), works on every
-        space).  Nothing but a few scalars crosses PCIe.  w_dev: n_cols doubles (state in / solution out)."""
+        "basic" (full steps).  ``pc``: the preconditioner of the TFQMR solves, as in ``tfqmr`` (6 and 7, the point ILU(0)s, work on
+        every space).  Nothing but a few scalars crosses PCIe.  w_dev: n_cols doubles (state in / solution out)."""
         nbytes = 8 * self.n_cols
         owns = work is None
         F_dev, dw_dev = (self.dev_alloc(nbytes), self.dev_alloc(nbytes)) if owns else work[:2]

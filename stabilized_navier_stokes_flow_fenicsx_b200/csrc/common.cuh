@@ -94,6 +94,7 @@ struct nsgpu_ctx {
   void* krylov = nullptr;                      // work vectors of the device-resident TFQMR (krylov.cu)
   void* ilu = nullptr;                         // colouring + factors of the multicolour block ILU(0) preconditioner (ilu.cu)
   void* pilu = nullptr;                        // colouring + factor of the multicolour point ILU(0) preconditioner (pilu.cu)
+  void* nilu = nullptr;                        // factor of the point ILU(0) in the caller's order (nilu.cu)
   void* rowown_plan = nullptr;                 // entity incidence lists + point records of the row-owner kernel (rowown.cu)
   void* trace = nullptr;                       // velocity tables of the streamline tracer (streamtrace.cu)
   nsgpu::Locator* locator = nullptr;           // point locator of the mesh (locate.cu)
@@ -242,6 +243,13 @@ bool pilu_factored(const nsgpu_ctx* ctx);
 int pilu_apply(nsgpu_ctx* ctx, const double* d_r, double* d_z);
 int pilu_colours(nsgpu_ctx* ctx, int32_t* h_colour, int32_t* n_colours, int32_t* n_vel_colours);
 void pilu_free(nsgpu_ctx* ctx);
+// nilu.cu
+int nilu_factor(nsgpu_ctx* ctx);
+bool nilu_factored(const nsgpu_ctx* ctx);
+int nilu_apply(nsgpu_ctx* ctx, const double* d_r, double* d_z);
+int nilu_status(nsgpu_ctx* ctx);
+int nilu_depth(nsgpu_ctx* ctx, int32_t* depth_lower, int32_t* depth_upper);
+void nilu_free(nsgpu_ctx* ctx);
 // rowown.cu
 bool rowown_available(nsgpu_ctx* ctx);
 int rowown_assemble(nsgpu_ctx* ctx, const double* d_xin, bool want_J, bool want_F, double* d_Fout);

@@ -286,6 +286,7 @@ static int reduce_and_update(nsgpu_ctx* ctx, Work& k, int nblocks, int what) {
 static int pc_apply(nsgpu_ctx* ctx, Work& k, int bs, const double* y, double* t) {
   if (bs == 5) return ilu_apply(ctx, y, t);                       // multicolour block ILU(0), ilu.cu
   if (bs == 6) return pilu_apply(ctx, y, t);                      // multicolour point ILU(0), pilu.cu
+  if (bs == 7) return nilu_apply(ctx, y, t);                      // point ILU(0) in the caller's order, nilu.cu
   const bool wide = bs == 4 && ((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(k.dinv)) & 31) == 0;
   k_pc_apply<<<(unsigned)ceil_div(k.n > 0 ? k.n : 1, 256), 256, 0, ctx->stream>>>(k.n, bs, k.dinv, y, t, wide);
   ctx->launches += 1;
@@ -314,14 +315,17 @@ int tfqmr_impl(nsgpu_ctx* ctx, const double* d_b, double* d_x, double rtol, doub
   const unsigned g = vgrid(n);
   int bs = pc;
   if (bs == 4 && (n % 4 != 0 || ctx->gdim != 3 || ctx->vdeg != 1)) bs = 1;   // vertex blocks only exist for P1-P1 tets
-  if (bs != 0 && bs != 1 && bs != 4 && bs != 5 && bs != 6) {
-    set_error(ctx, "tfqmr: pc must be 0 (none), 1 (Jacobi), 4 (4x4 block Jacobi), 5 (multicolour block ILU(0)) or 6 (multicolour point ILU(0))");
+  if (bs != 0 && bs != 1 && bs != 4 && bs != 5 && bs != 6 && bs != 7) {
+    set_error(ctx, "tfqmr: pc must be 0 (none), 1 (Jacobi), 4 (4x4 block Jacobi), 5 (multicolour block ILU(0)), 6 (multicolour point ILU(0)) "
+                   "or 7 (point ILU(0) in the caller's order)");
     return NSGPU_EINVAL;
   }
   if (bs == 5) {
     if ((rc = ilu_factor(ctx))) return rc;
   } else if (bs == 6) {
     if ((rc = pilu_factor(ctx))) return rc;
+  } else if (bs == 7) {
+    if ((rc = nilu_factor(ctx))) return rc;
   } else if (bs) {
     const int64_t ne = bs == 4 ? n / 4 : n;
     k_pc_setup<<<(unsigned)ceil_div(ne > 0 ? ne : 1, 128), 128, 0, s>>>(n, bs, ctx->d_indptr, ctx->d_indices, ctx->d_diag, ctx->d_vals, k.dinv);
@@ -393,6 +397,7 @@ int tfqmr_impl(nsgpu_ctx* ctx, const double* d_b, double* d_x, double rtol, doub
   NS_CUDA(ctx, cudaMemcpyAsync(&red, k.scal + S_RED, sizeof(double), cudaMemcpyDeviceToHost, s));
   NS_CUDA(ctx, cudaStreamSynchronize(s));
   NS_CUDA(ctx, cudaGetLastError());
+  if (bs == 7 && (rc = nilu_status(ctx))) return rc;
   if (its_out) *its_out = its;
   if (rnorm_out) *rnorm_out = sqrt(red);
   return NSGPU_OK;

@@ -152,6 +152,7 @@ int nsgpu_destroy(nsgpu_ctx* ctx) {
   krylov_free(ctx);
   ilu_free(ctx);
   pilu_free(ctx);
+  nilu_free(ctx);
   rowown_free(ctx);
   trace_free(ctx);
   locator_free(ctx);
@@ -604,6 +605,26 @@ int nsgpu_pilu_colours(nsgpu_ctx* ctx, int32_t* colour, int32_t* n_colours, int3
   NS_ENTER(ctx);
   NS_REQUIRE(ctx, ctx->pattern_built, "pilu_colours: call build_pattern first");
   return pilu_colours(ctx, colour, n_colours, n_velocity_colours);
+}
+
+int nsgpu_nilu_apply(nsgpu_ctx* ctx, int refactor, const double* r_owned, double* z_owned) {
+  NS_ENTER(ctx);
+  NS_REQUIRE(ctx, ctx->pattern_built, "nilu_apply: call build_pattern and assemble a Jacobian first");
+  NS_REQUIRE(ctx, r_owned && z_owned, "nilu_apply: NULL argument");
+  int rc;
+  if ((refactor || !nilu_factored(ctx)) && (rc = nilu_factor(ctx))) return rc;
+  if ((rc = vec_in(ctx, r_owned, ctx->d_F, ctx->n_owned))) return rc;
+  if ((rc = nilu_apply(ctx, ctx->d_F, ctx->d_F))) return rc;
+  if ((rc = nilu_status(ctx))) return rc;
+  if ((rc = vec_out(ctx, ctx->d_F, z_owned, ctx->n_owned))) return rc;
+  NS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return NSGPU_OK;
+}
+
+int nsgpu_nilu_depth(nsgpu_ctx* ctx, int32_t* depth_lower, int32_t* depth_upper) {
+  NS_ENTER(ctx);
+  NS_REQUIRE(ctx, ctx->pattern_built, "nilu_depth: call build_pattern first");
+  return nilu_depth(ctx, depth_lower, depth_upper);
 }
 
 int nsgpu_axpy_dev(nsgpu_ctx* ctx, double a, const double* x_dev, double* y_dev) {

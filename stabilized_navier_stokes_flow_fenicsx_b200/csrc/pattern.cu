@@ -346,6 +346,7 @@ int build_pattern_impl(nsgpu_ctx* ctx) {
   rowown_free(ctx);
   ilu_free(ctx);
   pilu_free(ctx);
+  nilu_free(ctx);
   cleanup();
   if (bad) {
     set_error(ctx, "build_pattern: a cell dof is missing from its row, or a row holds more than 65535 entries");

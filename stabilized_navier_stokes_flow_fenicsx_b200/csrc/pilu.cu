@@ -17,10 +17,11 @@
 //   apply       z = U^-1 L^-1 r: one launch per colour forwards, one per colour backwards, LPR lanes per row as in the CSR SpMV
 //
 // The factor lives in a packed copy in elimination order (per row its L entries, then its U entries, column inline), so the rows
-// of one colour are one contiguous stream of 12 bytes per entry: an application reads what one CSR SpMV reads.
+// of one colour are one contiguous stream of 12 bytes per entry: an application reads what one CSR SpMV reads.  The layout and the
+// per-row update are shared with the caller's-order ILU(0) of nilu.cu (pc = 7) through pilu_core.cuh.
 #include <cub/cub.cuh>
 
-#include "common.cuh"
+#include "pilu_core.cuh"
 
 namespace nsgpu {
 
@@ -31,16 +32,12 @@ struct PiluPlan {
   int n_colours = 0, n_vel_colours = 0;
   std::vector<int64_t> cstart;      // n_colours + 1 offsets into the elimination order
   int32_t* d_colour = nullptr;      // per owned row (internal numbering)
-  int4* d_erec = nullptr;           // per position of the order: (row, nL | nU << 16, first packed entry lo, hi)
-  int64_t* d_emap = nullptr;        // packed entry -> CSR position (its source in d_lu)
-  int32_t* d_ecol = nullptr;        // packed entry -> column
+  PackedLayout L;                   // keyed by colour
   double* d_lue = nullptr;          // packed factor values
   double* d_lu = nullptr;           // factor in CSR positions of the owned rows (workspace of the factorisation)
   double* d_uinv = nullptr;         // per owned row: 1 / u_ii
   int* d_bad = nullptr;             // smallest row with a zero / non-finite pivot (INT_MAX: none)
   double* d_flag = nullptr;         // the same as a count, reduced over the ranks
-  int64_t n_packed = 0, nnz_owned = 0;
-  int lpr = 4;                      // lanes per row of the sweeps
   bool factored = false;            // d_lue / d_uinv hold a usable factorisation of the current values
 };
 
@@ -53,27 +50,27 @@ __global__ void k_pilu_classify(int64_t n_cells, int nd, int first_p, int64_t n_
   if (d >= 0 && d < n_owned) isp[d] = 1;
 }
 
-// per position of the elimination order: its row and the sizes of its L (earlier colour) and U (later colour) parts
+// per position of the elimination order: its row and the sizes of its L (smaller key) and U (larger key) parts
 __global__ void k_pilu_count(int64_t n, const int32_t* __restrict__ order, const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices,
-                             const int32_t* __restrict__ colour, int4* erec, int64_t* cnt) {
+                             const int32_t* __restrict__ key, int4* erec, int64_t* cnt) {
   const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (idx > n) return;
   if (idx == n) { cnt[idx] = 0; return; }
   const int64_t i = order[idx];
-  const int c = colour[i];
+  const int c = key[i];
   int nL = 0, nU = 0;
   for (int64_t p = indptr[i]; p < indptr[i + 1]; ++p) {
     const int64_t j = indices[p];
     if (j >= n || j == i) continue;
-    if (colour[j] < c) ++nL; else ++nU;
+    if (key[j] < c) ++nL; else ++nU;
   }
   erec[idx] = make_int4((int)i, nL | (nU << 16), 0, 0);
   cnt[idx] = nL + nU;
 }
 
-// packed entries of each position in CSR order, keyed by (colour of the column, column): sorted per row, the L part comes first
+// packed entries of each position in CSR order, keyed by (key of the column, column): sorted per row, the L part comes first
 // in elimination order, then the U part
-__global__ void k_pilu_fill(int64_t n, const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices, const int32_t* __restrict__ colour,
+__global__ void k_pilu_fill(int64_t n, const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices, const int32_t* __restrict__ key,
                             const int64_t* __restrict__ eoff, int4* erec, uint64_t* ekey, int64_t* epos) {
   const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (idx >= n) return;
@@ -85,7 +82,7 @@ __global__ void k_pilu_fill(int64_t n, const int64_t* __restrict__ indptr, const
   for (int64_t p = indptr[i]; p < indptr[i + 1]; ++p) {
     const int64_t j = indices[p];
     if (j >= n || j == i) continue;
-    ekey[q] = ((uint64_t)(uint32_t)colour[j] << 32) | (uint64_t)j;
+    ekey[q] = ((uint64_t)(uint32_t)key[j] << 32) | (uint64_t)j;
     epos[q] = p;
     ++q;
   }
@@ -96,8 +93,7 @@ __global__ void k_pilu_ecol(int64_t np, const uint64_t* __restrict__ ekey, int32
   if (q < np) ecol[q] = (int32_t)(ekey[q] & 0xffffffffu);
 }
 
-// factorise the rows at positions [i0, i1) of the order (one colour) in place in lu (CSR positions).  One warp per row: the steps
-// over the earlier neighbours k are sequential, the updates of the row's later entries j are spread over the lanes.
+// factorise the rows at positions [i0, i1) of the order (one colour) in place in lu (CSR positions), one warp per row
 __global__ void __launch_bounds__(256)
 k_pilu_factor(int64_t i0, int64_t i1, int64_t n, const int4* __restrict__ erec, const int64_t* __restrict__ emap, const int32_t* __restrict__ ecol,
               const int32_t* __restrict__ colour, const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices,
@@ -107,38 +103,8 @@ k_pilu_factor(int64_t i0, int64_t i1, int64_t n, const int4* __restrict__ erec, 
   if (idx >= i1) return;                                     // uniform over the warp
   const int4 rec = erec[idx];
   const int64_t i = rec.x;
-  const int nL = rec.y & 0xffff;
   const int64_t q0 = (int64_t)(uint32_t)rec.z | ((int64_t)rec.w << 32);
-  const int64_t b = indptr[i], e = indptr[i + 1];
-  for (int t = 0; t < nL; ++t) {
-    const int64_t pk = emap[q0 + t];
-    const int64_t k = ecol[q0 + t];
-    const double l = lu[pk] * uinv[k];                       // a_ik / u_kk
-    const int ck = colour[k];
-    const int64_t kb = indptr[k], ke = indptr[k + 1];
-    for (int64_t p = b + lane; p < e; p += 32) {
-      const int32_t j = indices[p];
-      if (j >= n || colour[j] <= ck) continue;               // other rank's column, k itself, or an entry eliminated before k
-      int64_t lo = kb, hi = ke - 1, u = -1;                  // (k, j) in row k?  columns are sorted
-      while (lo <= hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        const int32_t cm = indices[mid];
-        if (cm == j) { u = mid; break; }
-        if (cm < j) lo = mid + 1; else hi = mid - 1;
-      }
-      if (u >= 0) lu[p] -= l * lu[u];
-    }
-    __syncwarp();
-    if (lane == 0) lu[pk] = l;                               // no lane reads a_ik again: later steps skip columns of colour <= ck
-  }
-  __syncwarp();
-  if (lane == 0) {
-    const int64_t d = diag[i];
-    const double piv = d >= 0 ? lu[d] : 0.0;
-    const bool ok = piv != 0.0 && isfinite(piv);
-    uinv[i] = ok ? 1.0 / piv : 0.0;
-    if (!ok) atomicMin(bad, (int)i);
-  }
+  if (pilu_factor_row(lane, i, rec.y & 0xffff, q0, n, emap, ecol, colour, indptr, indices, diag, lu, uinv, NoWait()) > 0) atomicMin(bad, (int)i);
 }
 
 __global__ void k_pilu_pack(int64_t np, const int64_t* __restrict__ emap, const double* __restrict__ lu, double* __restrict__ lue) {
@@ -171,16 +137,77 @@ k_pilu_sweep(int64_t i0, int64_t i1, const int4* __restrict__ erec, const int32_
   if (idx < i1 && lane == 0) z[i] = LOWER ? z[i] - s : uinv[i] * (z[i] - s);
 }
 
+void packed_layout_free(PackedLayout* L) {
+  cudaFree(L->d_erec); cudaFree(L->d_emap); cudaFree(L->d_ecol);
+  *L = PackedLayout();
+}
+
 void pilu_free(nsgpu_ctx* ctx) {
   PiluPlan* P = static_cast<PiluPlan*>(ctx->pilu);
   if (!P) return;
-  cudaFree(P->d_colour); cudaFree(P->d_erec); cudaFree(P->d_emap); cudaFree(P->d_ecol); cudaFree(P->d_lue); cudaFree(P->d_lu);
-  cudaFree(P->d_uinv); cudaFree(P->d_bad); cudaFree(P->d_flag);
+  packed_layout_free(&P->L);
+  cudaFree(P->d_colour); cudaFree(P->d_lue); cudaFree(P->d_lu); cudaFree(P->d_uinv); cudaFree(P->d_bad); cudaFree(P->d_flag);
   delete P;
   ctx->pilu = nullptr;
 }
 
 static inline unsigned pg256(int64_t n) { return (unsigned)ceil_div(n > 0 ? n : 1, 256); }
+
+int packed_layout(nsgpu_ctx* ctx, const char* who, int64_t n, const int32_t* d_order, const int32_t* d_key, PackedLayout* L) {
+  packed_layout_free(L);
+  cudaStream_t s = ctx->stream;
+  uint64_t *d_ekey = nullptr, *d_ekey2 = nullptr;
+  int64_t *d_cnt = nullptr, *d_eoff = nullptr, *d_epos = nullptr;
+  void* d_tmp = nullptr;
+  auto done = [&](int rc, const std::string& msg) {
+    if (!msg.empty()) set_error(ctx, std::string(who) + ": " + msg);
+    cudaFree(d_ekey); cudaFree(d_ekey2); cudaFree(d_cnt); cudaFree(d_eoff); cudaFree(d_epos); cudaFree(d_tmp);
+    if (rc) packed_layout_free(L);
+    return rc;
+  };
+#define PL_CUDA(call)                                                                              \
+  do {                                                                                             \
+    cudaError_t e__ = (call);                                                                      \
+    if (e__ != cudaSuccess) return done(NSGPU_ECUDA, std::string(#call ": ") + cudaGetErrorString(e__)); \
+  } while (0)
+  PL_CUDA(cudaMalloc(&L->d_erec, sizeof(int4) * n));
+  PL_CUDA(cudaMalloc(&d_cnt, sizeof(int64_t) * (n + 1)));
+  PL_CUDA(cudaMalloc(&d_eoff, sizeof(int64_t) * (n + 1)));
+  k_pilu_count<<<pg256(n + 1), 256, 0, s>>>(n, d_order, ctx->d_indptr, ctx->d_indices, d_key, L->d_erec, d_cnt);
+  size_t tb = 0;
+  PL_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb, d_cnt, d_eoff, n + 1, s));
+  PL_CUDA(cudaMalloc(&d_tmp, tb));
+  PL_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tb, d_cnt, d_eoff, n + 1, s));
+  cudaFree(d_tmp); d_tmp = nullptr;
+  int64_t np = 0;
+  PL_CUDA(cudaMemcpyAsync(&np, d_eoff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+  PL_CUDA(cudaMemcpyAsync(&L->nnz_owned, ctx->d_indptr + n, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+  PL_CUDA(cudaStreamSynchronize(s));
+  ctx->launches += 2;
+  if (np >= (int64_t(1) << 31)) return done(NSGPU_EUNSUPPORTED, "more than 2^31 owned off-diagonal entries on one rank");
+  L->n_packed = np;
+  PL_CUDA(cudaMalloc(&d_ekey, sizeof(uint64_t) * (np > 0 ? np : 1)));
+  PL_CUDA(cudaMalloc(&d_ekey2, sizeof(uint64_t) * (np > 0 ? np : 1)));
+  PL_CUDA(cudaMalloc(&d_epos, sizeof(int64_t) * (np > 0 ? np : 1)));
+  PL_CUDA(cudaMalloc(&L->d_emap, sizeof(int64_t) * (np > 0 ? np : 1)));
+  PL_CUDA(cudaMalloc(&L->d_ecol, sizeof(int32_t) * (np > 0 ? np : 1)));
+  k_pilu_fill<<<pg256(n), 256, 0, s>>>(n, ctx->d_indptr, ctx->d_indices, d_key, d_eoff, L->d_erec, d_ekey, d_epos);
+  ctx->launches += 1;
+  if (np > 0) {
+    PL_CUDA(cub::DeviceSegmentedSort::SortPairs(nullptr, tb, d_ekey, d_ekey2, d_epos, L->d_emap, (int)np, (int)n, d_eoff, d_eoff + 1, s));
+    PL_CUDA(cudaMalloc(&d_tmp, tb));
+    PL_CUDA(cub::DeviceSegmentedSort::SortPairs(d_tmp, tb, d_ekey, d_ekey2, d_epos, L->d_emap, (int)np, (int)n, d_eoff, d_eoff + 1, s));
+    k_pilu_ecol<<<pg256(np), 256, 0, s>>>(np, d_ekey2, L->d_ecol);
+    ctx->launches += 2;
+  }
+  PL_CUDA(cudaStreamSynchronize(s));
+  PL_CUDA(cudaGetLastError());
+#undef PL_CUDA
+  // lanes per row of the sweeps from the mean length of a row's L or U part (the CSR SpMV's rule on whole rows)
+  const double avg = (double)np / (double)n;
+  L->lpr = avg > 48 ? 16 : (avg > 24 ? 8 : 4);
+  return done(NSGPU_OK, "");
+}
 
 // classes, colouring, elimination order and the packed layout of the factor (once per pattern)
 static int pilu_plan(nsgpu_ctx* ctx) {
@@ -193,12 +220,9 @@ static int pilu_plan(nsgpu_ctx* ctx) {
   P->n = n;
   uint8_t* d_isp = nullptr;
   int32_t* d_order = nullptr;
-  uint64_t *d_ekey = nullptr, *d_ekey2 = nullptr;
-  int64_t *d_cnt = nullptr, *d_eoff = nullptr, *d_epos = nullptr;
-  void* d_tmp = nullptr;
   auto done = [&](int rc, const std::string& msg) {   // msg empty: the callee has set the message
     if (!msg.empty()) set_error(ctx, msg);
-    cudaFree(d_isp); cudaFree(d_order); cudaFree(d_ekey); cudaFree(d_ekey2); cudaFree(d_cnt); cudaFree(d_eoff); cudaFree(d_epos); cudaFree(d_tmp);
+    cudaFree(d_isp); cudaFree(d_order);
     if (rc) pilu_free(ctx);
     return rc;
   };
@@ -217,47 +241,13 @@ static int pilu_plan(nsgpu_ctx* ctx) {
   // velocity rows (class 0) from colour 0, then pressure rows (class 1) from the first colour after the velocity ones
   if (int rc = mc_colour(ctx, n, 0, d_isp, PILU_MAX_COLOURS, "pc = 6", P->d_colour, d_order, P->cstart, &P->n_vel_colours)) return done(rc, "");
   P->n_colours = (int)P->cstart.size() - 1;
-  // the packed layout
-  PL_CUDA(cudaMalloc(&P->d_erec, sizeof(int4) * n));
-  PL_CUDA(cudaMalloc(&d_cnt, sizeof(int64_t) * (n + 1)));
-  PL_CUDA(cudaMalloc(&d_eoff, sizeof(int64_t) * (n + 1)));
-  k_pilu_count<<<pg256(n + 1), 256, 0, s>>>(n, d_order, ctx->d_indptr, ctx->d_indices, P->d_colour, P->d_erec, d_cnt);
-  size_t tb = 0;
-  PL_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb, d_cnt, d_eoff, n + 1, s));
-  PL_CUDA(cudaMalloc(&d_tmp, tb));
-  PL_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tb, d_cnt, d_eoff, n + 1, s));
-  cudaFree(d_tmp); d_tmp = nullptr;
-  int64_t np = 0;
-  PL_CUDA(cudaMemcpyAsync(&np, d_eoff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
-  PL_CUDA(cudaMemcpyAsync(&P->nnz_owned, ctx->d_indptr + n, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
-  PL_CUDA(cudaStreamSynchronize(s));
-  ctx->launches += 2;
-  if (np >= (int64_t(1) << 31)) return done(NSGPU_EUNSUPPORTED, "pc = 6: more than 2^31 owned off-diagonal entries on one rank");
-  P->n_packed = np;
-  PL_CUDA(cudaMalloc(&d_ekey, sizeof(uint64_t) * (np > 0 ? np : 1)));
-  PL_CUDA(cudaMalloc(&d_ekey2, sizeof(uint64_t) * (np > 0 ? np : 1)));
-  PL_CUDA(cudaMalloc(&d_epos, sizeof(int64_t) * (np > 0 ? np : 1)));
-  PL_CUDA(cudaMalloc(&P->d_emap, sizeof(int64_t) * (np > 0 ? np : 1)));
-  PL_CUDA(cudaMalloc(&P->d_ecol, sizeof(int32_t) * (np > 0 ? np : 1)));
+  if (int rc = packed_layout(ctx, "pc = 6", n, d_order, P->d_colour, &P->L)) return done(rc, "");
+  const int64_t np = P->L.n_packed;
   PL_CUDA(cudaMalloc(&P->d_lue, sizeof(double) * (np > 0 ? np : 1)));
-  PL_CUDA(cudaMalloc(&P->d_lu, sizeof(double) * (P->nnz_owned > 0 ? P->nnz_owned : 1)));
+  PL_CUDA(cudaMalloc(&P->d_lu, sizeof(double) * (P->L.nnz_owned > 0 ? P->L.nnz_owned : 1)));
   PL_CUDA(cudaMalloc(&P->d_uinv, sizeof(double) * n));
   PL_CUDA(cudaMalloc(&P->d_bad, sizeof(int)));
   PL_CUDA(cudaMalloc(&P->d_flag, sizeof(double)));
-  k_pilu_fill<<<pg256(n), 256, 0, s>>>(n, ctx->d_indptr, ctx->d_indices, P->d_colour, d_eoff, P->d_erec, d_ekey, d_epos);
-  ctx->launches += 1;
-  if (np > 0) {
-    PL_CUDA(cub::DeviceSegmentedSort::SortPairs(nullptr, tb, d_ekey, d_ekey2, d_epos, P->d_emap, (int)np, (int)n, d_eoff, d_eoff + 1, s));
-    PL_CUDA(cudaMalloc(&d_tmp, tb));
-    PL_CUDA(cub::DeviceSegmentedSort::SortPairs(d_tmp, tb, d_ekey, d_ekey2, d_epos, P->d_emap, (int)np, (int)n, d_eoff, d_eoff + 1, s));
-    k_pilu_ecol<<<pg256(np), 256, 0, s>>>(np, d_ekey2, P->d_ecol);
-    ctx->launches += 2;
-  }
-  PL_CUDA(cudaStreamSynchronize(s));
-  PL_CUDA(cudaGetLastError());
-  // lanes per row of the sweeps from the mean length of a row's L or U part (the CSR SpMV's rule on whole rows)
-  const double avg = (double)np / (double)n;
-  P->lpr = avg > 48 ? 16 : (avg > 24 ? 8 : 4);
 #undef PL_CUDA
   return done(NSGPU_OK, "");
 }
@@ -272,15 +262,15 @@ int pilu_factor(nsgpu_ctx* ctx) {
   }
   cudaStream_t s = ctx->stream;
   P->factored = false;
-  NS_CUDA(ctx, cudaMemcpyAsync(P->d_lu, ctx->d_vals, sizeof(double) * (size_t)P->nnz_owned, cudaMemcpyDeviceToDevice, s));
+  NS_CUDA(ctx, cudaMemcpyAsync(P->d_lu, ctx->d_vals, sizeof(double) * (size_t)P->L.nnz_owned, cudaMemcpyDeviceToDevice, s));
   NS_CUDA(ctx, cudaMemsetAsync(P->d_bad, 0x7f, sizeof(int), s));
   for (int c = 0; c < P->n_colours; ++c) {
     const int64_t i0 = P->cstart[c], i1 = P->cstart[c + 1];
     if (i1 == i0) continue;
-    k_pilu_factor<<<(unsigned)ceil_div(i1 - i0, 8), 256, 0, s>>>(i0, i1, P->n, P->d_erec, P->d_emap, P->d_ecol, P->d_colour, ctx->d_indptr,
+    k_pilu_factor<<<(unsigned)ceil_div(i1 - i0, 8), 256, 0, s>>>(i0, i1, P->n, P->L.d_erec, P->L.d_emap, P->L.d_ecol, P->d_colour, ctx->d_indptr,
                                                                   ctx->d_indices, ctx->d_diag, P->d_lu, P->d_uinv, P->d_bad);
   }
-  k_pilu_pack<<<pg256(P->n_packed), 256, 0, s>>>(P->n_packed, P->d_emap, P->d_lu, P->d_lue);
+  k_pilu_pack<<<pg256(P->L.n_packed), 256, 0, s>>>(P->L.n_packed, P->L.d_emap, P->d_lu, P->d_lue);
   ctx->launches += P->n_colours + 1;
   NS_CUDA(ctx, cudaGetLastError());
   int bad = 0;
@@ -319,11 +309,11 @@ int pilu_apply(nsgpu_ctx* ctx, const double* d_r, double* d_z) {
   if (d_z != d_r) NS_CUDA(ctx, cudaMemcpyAsync(d_z, d_r, sizeof(double) * (size_t)P->n, cudaMemcpyDeviceToDevice, s));
   auto sweep = [&](int c, bool lower) {
     const int64_t i0 = P->cstart[c], i1 = P->cstart[c + 1];
-    const unsigned g = pg256((i1 - i0) * P->lpr);
-#define PILU_SWEEP(L)                                                                                                   \
-    if (lower) k_pilu_sweep<L, true><<<g, 256, 0, s>>>(i0, i1, P->d_erec, P->d_ecol, P->d_lue, P->d_uinv, d_z);        \
-    else k_pilu_sweep<L, false><<<g, 256, 0, s>>>(i0, i1, P->d_erec, P->d_ecol, P->d_lue, P->d_uinv, d_z);
-    if (P->lpr == 16) { PILU_SWEEP(16) } else if (P->lpr == 8) { PILU_SWEEP(8) } else { PILU_SWEEP(4) }
+    const unsigned g = pg256((i1 - i0) * P->L.lpr);
+#define PILU_SWEEP(LPR)                                                                                                   \
+    if (lower) k_pilu_sweep<LPR, true><<<g, 256, 0, s>>>(i0, i1, P->L.d_erec, P->L.d_ecol, P->d_lue, P->d_uinv, d_z);        \
+    else k_pilu_sweep<LPR, false><<<g, 256, 0, s>>>(i0, i1, P->L.d_erec, P->L.d_ecol, P->d_lue, P->d_uinv, d_z);
+    if (P->L.lpr == 16) { PILU_SWEEP(16) } else if (P->L.lpr == 8) { PILU_SWEEP(8) } else { PILU_SWEEP(4) }
 #undef PILU_SWEEP
   };
   for (int c = 1; c < P->n_colours; ++c) sweep(c, true);      // colour 0 has no earlier neighbour
